@@ -30,6 +30,8 @@ the max-over-ranks only.
              fragments, seed 0x5EED0003), each with its own roofline fraction and a sample checked against the CPU reference.
 `cpu_baseline` the unmodified reference (oracle/_ref) or the oracle port on this box's cores.
 --impl reference times that CPU implementation alone (same config, same protocol: oracle.BatchRunner.measure).
+--dump-outputs DIR writes what the last timed step returned (rank 0's pages) as .npy files, see dump_outputs();
+             the inputs depend on the arguments only, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -170,6 +172,32 @@ def run_reference(args, rank: int, world: int):
         "gpu_launches": 0,
     }
     print(json.dumps(line), flush=True)
+
+
+def dump_outputs(path: str, B: int, ostride: int, comp, comp_len, back, back_len, status):
+    """The results of the timed step as float32 .npy files under `path` (57 MB at most), on pages picked by a fixed
+    seed: compressed_len / decompressed_len / status of up to 1 Mi pages (all pages of the default batch; their
+    indices in len_pages.npy) and compressed / decompressed bytes of 1024 pages (indices in byte_pages.npy).  A
+    compressed slot is zeroed past its length: those bytes are not part of the result."""
+    import numpy as np
+    import torch
+
+    os.makedirs(path, exist_ok=True)
+    rng = np.random.default_rng(0x5EED0D)
+    len_pages = np.sort(rng.choice(B, min(B, 1 << 20), replace=False))
+    byte_pages = np.sort(rng.choice(B, min(B, 1024), replace=False))
+    li = torch.from_numpy(len_pages).to(comp.device)
+    bi = torch.from_numpy(byte_pages).to(comp.device)
+    c = comp.view(B, ostride).index_select(0, bi).float()
+    c *= torch.arange(ostride, device=c.device)[None, :] < comp_len.index_select(0, bi)[:, None]
+    out = {"len_pages": len_pages.astype(np.float64), "byte_pages": byte_pages.astype(np.float64),
+           "compressed_len": comp_len.index_select(0, li), "decompressed_len": back_len.index_select(0, li),
+           "status": status.index_select(0, li), "compressed": c,
+           "decompressed": back.view(B, PAGE).index_select(0, bi)}
+    for name, a in out.items():
+        if isinstance(a, torch.Tensor):
+            a = a.float().cpu().numpy()
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def run_workloads(args, cs, synth, dev, rank, world, barrier):
@@ -321,7 +349,11 @@ def main():
     ap.add_argument("--wave-gib", type=float, default=16.0, help="decode_only: GiB per wave")
     ap.add_argument("--only", default="", choices=["", "text", "zero", "random"],
                     help="diagnostic: make every page of one class (not the BASELINE workload)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step computed (rank 0's pages) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -407,6 +439,8 @@ def main():
     elapsed_ms = t0.elapsed_time(t1)
     tc_ms = statistics.mean(e[0].elapsed_time(e[1]) for e in evs)
     td_ms = statistics.mean(e[1].elapsed_time(e[2]) for e in evs)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, B, ostride, comp, comp_len, back, back_len, status)
 
     # ---- e2e through the host-buffer C-ABI with pinned host memory ------------------------
     # The call a block_compressor / zram style user makes: pages in host memory -> the page container

@@ -32,6 +32,7 @@
 //     memory instead (Input<false>): only the table stays in shared memory, 7 chains per SM.
 #include <stdlib.h>
 
+#include <mutex>
 #include <type_traits>
 
 #include "device_common.cuh"
@@ -684,6 +685,10 @@ using namespace csb;
 template <int G, bool ST>
 static int launch_compress_g(const CompressParams &p, int threads, int ctas, size_t smem, cudaStream_t s)
 {
+	// The attributes belong to the kernel, not to the launch: a concurrent caller that set a smaller shared-memory
+	// limit between our set and our launch would make the launch fail.  Set and launch as one step.
+	static std::mutex mu;
+	std::lock_guard<std::mutex> lk(mu);
 	cudaError_t e = cudaFuncSetAttribute(compress_kernel<G, ST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
 	if (e != cudaSuccess)
 		return (int)e;

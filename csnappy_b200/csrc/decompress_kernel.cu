@@ -27,6 +27,8 @@
 //              of which fewer than 8 would fit per SM (32 KiB fragments): same three phases, but the input is
 //              read through L1 and the output lives in global memory, back-references through L2; no staging
 //              area, so every warp of the CTA runs its own block and the L2 latency is hidden by their number.
+#include <mutex>
+
 #include "device_common.cuh"
 #include "kernels.h"
 
@@ -693,6 +695,9 @@ using namespace csb;
 template <int G, bool GIN>
 static int launch_decompress_gi(const DecompressParams &p, int threads, int ctas, size_t smem, cudaStream_t s)
 {
+	// set the kernel's attributes and launch as one step (see launch_compress_g)
+	static std::mutex mu;
+	std::lock_guard<std::mutex> lk(mu);
 	cudaError_t e = cudaFuncSetAttribute(decompress_kernel<G, GIN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
 	if (e != cudaSuccess)
 		return (int)e;

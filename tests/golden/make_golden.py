@@ -1,10 +1,11 @@
 #!/usr/bin/env python
 """Regenerate tests/golden/ from the UNMODIFIED reference.
 
-Run in the build container only (needs /root/reference and the reference
-compiled by oracle/Makefile into oracle/_ref/libcsnappy_ref.so):
+Needs the reference's sources (REF of oracle/Makefile) compiled by oracle/Makefile
+into oracle/_ref/libcsnappy_ref.so:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py           # everything below
+    python tests/golden/make_golden.py --cases   # reference_cases.json alone
 
 What it writes
   * gzip copies of the reference's own fixtures (data, not source):
@@ -14,7 +15,11 @@ What it writes
     seeded synthetic inputs -- sizes + sha256 of compressed streams for
     wm 9..16, per-fragment streams (4 KiB/13, 32 KiB/15, 32 KiB/16), the tiny
     input pins of SURVEY.md 8c, and the appendix-B decode matrix.
-The GPU box has no /root/reference; tests read only what is committed here.
+  * reference_cases.json: sha256 of the reference's results on the fuzz, edge-size and
+    corrupted-stream inputs of tests/cases.py, as the tests compare them.  `--cases` records
+    them with oracle.best() and names the checker in the file: without the reference library
+    that is the port (oracle/snappy_oracle.c).
+Tests read only what is committed here.
 """
 import gzip
 import hashlib
@@ -28,6 +33,7 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "..", ".."))
+sys.path.insert(0, os.path.join(HERE, ".."))
 import oracle  # noqa: E402
 
 REF_DATA = "/root/reference/testdata"
@@ -152,7 +158,46 @@ def main():
     with open(os.path.join(HERE, "golden.json"), "w") as f:
         json.dump(G, f, indent=1, sort_keys=True)
     print("wrote", os.path.join(HERE, "golden.json"))
+    write_reference_cases(ref)
+
+
+def write_reference_cases(chk):
+    """reference_cases.json: what tests/test_oracle.py and tests/test_gpu_canaries.py compare with."""
+    from cases import (CANARY_DECODE, EDGE_COMPRESS_SIZES, EDGE_FRAGMENT_SIZES, corrupt_streams, corrupted_fragments,
+                       edge_compress_input, edge_text, ends_inside_tag, ends_inside_tag_header, fuzz_pages)
+
+    def result(rc, out):
+        return [rc, None if out is None else sha(out)]
+
+    R = {"checker": chk.kind}
+    R["fuzz_fragments"] = {f"{size}/{wm}": [sha(chk.compress_fragment(p, wm)) for p in fuzz_pages(1234 + size + wm, 35, size)]
+                           for size, wm in ((4096, 13), (4096, 9), (32768, 15), (32768, 16), (1000, 12), (20000, 14))}
+    text = edge_text()
+    R["edge_fragments"] = {str(wm): [sha(chk.compress_fragment(text[:n], wm)) for n in EDGE_FRAGMENT_SIZES]
+                           for wm in (9, 13, 16)}
+    R["edge_compress"] = {str(wm): [sha(chk.compress(edge_compress_input(text, n), wm)) for n in EDGE_COMPRESS_SIZES]
+                          for wm in (9, 13, 15, 16)}
+    # the reference's x86 path is undefined on a stream cut inside a tag's trailing bytes: recorded as None
+    port = oracle.port()
+    R["corruptions"] = [None if port.decompress_noheader(d, cap)[0] == oracle.E_DATA_MALFORMED and ends_inside_tag(d)
+                        else result(*chk.decompress_noheader(d, cap)) for d, cap in corrupted_fragments(chk.compress_fragment)]
+    pages = np.frombuffer(b"".join(fuzz_pages(77, 64, 4096)), dtype=np.uint8).reshape(64, 4096)
+    out, out_len, _ = oracle.batch_compress(pages, 13, chk.kind, threads=2)
+    R["bulk_4096_13"] = {"len": out_len.tolist(), "sha256": [sha(out[i, : out_len[i]].tobytes()) for i in range(64)]}
+    R["canary_decode"] = {}
+    for (size, wm), (seed, count) in CANARY_DECODE.items():
+        streams, caps = corrupt_streams(chk.compress_fragment, size, wm, seed, count)
+        R["canary_decode"][f"{size}/{wm}"] = [None if ends_inside_tag_header(s) else result(*chk.decompress_noheader(s, cap))
+                                              for s, cap in zip(streams, caps)]
+    path = os.path.join(HERE, "reference_cases.json")
+    with open(path, "w") as f:
+        json.dump(R, f, indent=0, sort_keys=True)
+        f.write("\n")
+    print("wrote", path, "checker", chk.kind)
 
 
 if __name__ == "__main__":
-    main()
+    if "--cases" in sys.argv:
+        write_reference_cases(oracle.best())
+    else:
+        main()

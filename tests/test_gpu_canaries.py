@@ -9,14 +9,16 @@ untouched --
   compress  nothing past csnappy_max_compressed_length(n) (the reference REQUIRES that much room and
             checks nothing, cl_tester.c:120-165 -- the kernel must not need more).
 Also: corrupted streams that do NOT end inside a tag header are compared with the unmodified
-reference (oracle/_ref), not only with the port -- only the truncated-tag case is reference UB
-(SURVEY.md 0.5) and is defined here as -5.
+reference's results (tests/golden/reference_cases.json), not only with the port -- only the
+truncated-tag case is reference UB (SURVEY.md 0.5) and is defined here as -5.
 """
+import hashlib
+
 import numpy as np
 import pytest
 
 import oracle
-from cases import fuzz_pages
+from cases import CANARY_DECODE, corrupt_streams, fuzz_pages, reference_cases
 
 pytestmark = pytest.mark.gpu
 
@@ -34,59 +36,13 @@ def cs():
     return c
 
 
-def ends_inside_tag_header(s: bytes) -> bool:
-    """True when the end of input cuts a tag's header (tag byte + offset / length bytes): the reference's
-    UB case (csnappy_decompress.c:331-342,350).  Payload shortage of a literal is NOT that case (-5, :374)."""
-    pos, n = 0, len(s)
-    while pos < n:
-        tag = s[pos]
-        kind = tag & 3
-        if kind == 0:
-            ln = (tag >> 2) + 1
-            hdr = 1
-            if ln > 60:
-                nb = ln - 60
-                if pos + 1 + nb > n:
-                    return True
-                ln = int.from_bytes(s[pos + 1: pos + 1 + nb], "little") + 1
-                hdr = 1 + nb
-            pos += hdr + (ln & 0xFFFFFFFF)
-        else:
-            hdr = (2, 3, 5)[kind - 1]
-            if pos + hdr > n:
-                return True
-            pos += hdr
-    return False
-
-
-def _corrupt_streams(chk, size, wm, seed, count):
-    pages = fuzz_pages(seed, count, size)
-    comp = [chk.compress_fragment(p, wm) for p in pages]
-    rng = np.random.default_rng(seed + 1)
-    streams, caps = [], []
-    for i, c in enumerate(comp):
-        d = bytearray(c)
-        k = i % 6
-        if k == 1 and len(d) > 8:
-            d[int(rng.integers(0, len(d)))] ^= int(rng.integers(1, 256))
-        elif k == 2 and len(d) > 8:
-            d = d[: int(rng.integers(1, len(d)))]
-        elif k == 4 and len(d) > 8:
-            for _ in range(3):
-                d[int(rng.integers(0, len(d)))] = int(rng.integers(0, 256))
-        elif k == 5:
-            d += bytes(rng.integers(0, 256, int(rng.integers(1, 9)), dtype=np.uint8))
-        streams.append(bytes(d))
-        caps.append(size if k != 3 else int(rng.integers(1, size)))
-    return streams, caps
-
-
 @pytest.mark.parametrize("stage", [0, 2, 3, 4])
 @pytest.mark.parametrize("lanes", [32, 16, 8])
 @pytest.mark.parametrize("size,wm", [(4096, 13), (32768, 15)])
 def test_decode_never_writes_at_or_past_cap(cs, lanes, stage, size, wm):
-    chk = oracle.best()
-    streams, caps = _corrupt_streams(chk, size, wm, 515 + size, 84 if size == 4096 else 28)
+    streams, caps = corrupt_streams(oracle.best().compress_fragment, size, wm, *CANARY_DECODE[(size, wm)])
+    ref = reference_cases()["canary_decode"][f"{size}/{wm}"]
+    assert len(ref) == len(streams)
     B = len(streams)
     in_stride = (cs.csnappy_max_compressed_length(size) + 16 + 15) // 16 * 16
     out_stride = size + 256  # 256-byte guard band behind every slot
@@ -115,11 +71,11 @@ def test_decode_never_writes_at_or_past_cap(cs, lanes, stage, size, wm):
         assert (slot[caps[i]:] == PAT).all(), (i, "wrote at or past cap", caps[i], int(st[i]))
         rc, exp = oracle.port().decompress_noheader(s, caps[i])
         assert st[i] == rc, (i, s.hex()[:60])
-        if not ends_inside_tag_header(s) and oracle.have_reference():
-            rrc, rexp = oracle.reference().decompress_noheader(s, caps[i])
+        if ref[i] is not None:  # None: the stream ends inside a tag header
+            rrc, rsha = ref[i]
             assert (st[i], rc) == (rrc, rrc), (i, "differs from the unmodified reference", s.hex()[:60])
             if rrc == 0:
-                assert exp == rexp
+                assert hashlib.sha256(exp).hexdigest() == rsha
         if rc == 0:
             assert ol[i] == len(exp) and slot[: ol[i]].tobytes() == exp, i
         else:
