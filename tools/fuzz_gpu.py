@@ -1,6 +1,7 @@
 #!/usr/bin/env python
 """Long randomized parity run on the GPU box: many seeds / block sizes / table sizes / lane groups,
-compressed bytes and decoder results compared with the unmodified reference (oracle/_ref).
+compressed bytes and decoder results compared with the unmodified reference (oracle/_ref).  The decode leg
+also gets random streams of every tag form (tests/streams.py), which the compressor never writes.
 
     python tools/fuzz_gpu.py [seconds] [seed]
 """
@@ -15,6 +16,7 @@ sys.path.insert(0, "tests")
 import csnappy_b200 as cs
 import oracle
 from cases import fuzz_pages
+from streams import random_stream
 
 budget = float(sys.argv[1]) if len(sys.argv) > 1 else 120.0
 seed = int(sys.argv[2]) if len(sys.argv) > 2 else 20261017
@@ -65,13 +67,19 @@ while time.time() - t0 < budget:
         strs.append(bytes(d))
         caps.append(int(lens[i]) if k != 4 else int(rng.integers(0, max(1, int(lens[i])))))
     stride = (cs.csnappy_max_compressed_length(size) + 16 + 15) // 16 * 16
-    hs = np.zeros((count, stride), dtype=np.uint8)
-    sl = np.zeros(count, dtype=np.int32)
+    for _ in range(int(rng.integers(1, count // 4 + 2))):
+        s = random_stream(int(rng.integers(1 << 30)), int(rng.integers(1, size + 1)))
+        if len(s.buf) <= stride:  # capacity at most the block size: sometimes short of the stream's output
+            strs.append(bytes(s.buf))
+            caps.append(min(s.produced, size))
+    n_dec = len(strs)
+    hs = np.zeros((n_dec, stride), dtype=np.uint8)
+    sl = np.zeros(n_dec, dtype=np.int32)
     for i, s in enumerate(strs):
         hs[i, : len(s)] = np.frombuffer(s, dtype=np.uint8)
         sl[i] = len(s)
     ocap = (size + 15) // 16 * 16
-    res = cs.batch_decompress(torch.from_numpy(hs).cuda(), torch.from_numpy(sl).cuda(), count, size, in_stride=stride,
+    res = cs.batch_decompress(torch.from_numpy(hs).cuda(), torch.from_numpy(sl).cuda(), n_dec, size, in_stride=stride,
                               out_caps=torch.tensor(caps, dtype=torch.int32).cuda(), out_stride=max(ocap, 16))
     torch.cuda.synchronize()
     bo, bl, st = (x.cpu().numpy() for x in res)
@@ -80,7 +88,7 @@ while time.time() - t0 < budget:
         assert st[i] == rc, ("status", size, wm, lanes, i, int(st[i]), rc, s.hex()[:60])
         if rc == 0:
             assert bl[i] == len(exp) and bo[i * max(ocap, 16): i * max(ocap, 16) + bl[i]].tobytes() == exp, ("bytes", size, lanes, i)
-    streams += count
+    streams += n_dec
     rounds += 1
 cs.set_tuning("compress_lanes", 0)
 cs.set_tuning("decompress_lanes", 0)
