@@ -1,7 +1,9 @@
 #!/usr/bin/env python
 """Long randomized parity run on the GPU box: many seeds / block sizes / table sizes / lane groups,
-compressed bytes and decoder results compared with the unmodified reference (oracle/_ref).  The decode leg
-also gets random streams of every tag form (tests/streams.py), which the compressor never writes.
+compressed bytes and decoder results compared with the unmodified reference (oracle/_ref).  The compress leg
+also gets blocks built to drive the parse through the kernel's rare paths (tests/compress_cases.py: hash-slot
+sharing in stride-1 and strided windows, in-window copies, the scan end, length and offset boundaries); the decode
+leg gets random streams of every tag form (tests/streams.py), which the compressor never writes.
 
     python tools/fuzz_gpu.py [seconds] [seed]
 """
@@ -15,6 +17,7 @@ sys.path.insert(0, ".")
 sys.path.insert(0, "tests")
 import csnappy_b200 as cs
 import oracle
+import compress_cases
 from cases import fuzz_pages
 from streams import random_stream
 
@@ -30,6 +33,15 @@ while time.time() - t0 < budget:
     lanes = int(rng.choice([8, 16, 32]))
     count = int(rng.integers(20, 120))
     pages = fuzz_pages(int(rng.integers(1 << 30)), count, size)
+    if size >= 1000:  # a few constructed blocks per round (building one takes 0.1-1 s)
+        themes = ("share", "strided", "emit", "share")
+        for i in rng.choice(count, min(count, 3), replace=False):
+            try:
+                c = compress_cases.build_block(int(rng.integers(1 << 30)), size, wm, themes[int(i) % 4])
+            except compress_cases.Plan:
+                c = None
+            if c is not None:
+                pages[int(i)] = c.data
     # ragged lengths
     lens = np.array([int(rng.integers(0, size + 1)) if rng.random() < 0.3 else size for _ in pages], dtype=np.int32)
     host = np.zeros((count, size), dtype=np.uint8)
