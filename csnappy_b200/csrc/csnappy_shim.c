@@ -429,7 +429,7 @@ struct slot {
 	struct {
 		const void *src; /* pinned */
 		void *dst;	 /* the caller's pageable memory */
-		size_t n;
+		size_t width, pitch, rows; /* `rows` runs of `width` bytes, `pitch` apart on both sides */
 	} pend[3]; /* copies owed to the caller once the slot's queued device-to-host copies have landed */
 	int npend;
 	uint64_t first;
@@ -695,25 +695,50 @@ static int is_pageable(const void *p)
 	return at.type == cudaMemoryTypeUnregistered;
 }
 
-/* finish a slot's deferred copy-out: its device-to-host copies into the pinned staging have been queued on b->s */
-static void slot_owe(struct slot *b, const void *pinned_src, void *dst, size_t n)
+/* finish a slot's deferred copy-out: its device-to-host copies into the pinned staging have been queued on b->s.
+ * slot_owe2: `rows` runs of `width` bytes, `pitch` apart in the staging and in the caller's memory (the bytes in
+ * between belong to the caller and are not written). */
+static void slot_owe2(struct slot *b, const void *pinned_src, void *dst, size_t width, size_t pitch, size_t rows)
 {
 	b->pend[b->npend].src = pinned_src;
 	b->pend[b->npend].dst = dst;
-	b->pend[b->npend].n = n;
+	b->pend[b->npend].width = width;
+	b->pend[b->npend].pitch = pitch;
+	b->pend[b->npend].rows = rows;
 	b->npend++;
 }
+
+static void slot_owe(struct slot *b, const void *pinned_src, void *dst, size_t n) { slot_owe2(b, pinned_src, dst, n, n, 1); }
 
 static int slot_drain(struct slot *b)
 {
 	int e = 0, i;
+	size_t r;
 	if (!b->npend)
 		return 0;
 	e = (int)cudaStreamSynchronize(b->s);
-	for (i = 0; i < b->npend && !e; i++)
-		par_memcpy(b->pend[i].dst, b->pend[i].src, b->pend[i].n);
+	for (i = 0; i < b->npend && !e; i++) {
+		const uint8_t *s = (const uint8_t *)b->pend[i].src;
+		uint8_t *d = (uint8_t *)b->pend[i].dst;
+		if (b->pend[i].width == b->pend[i].pitch)
+			par_memcpy(d, s, b->pend[i].width * b->pend[i].rows);
+		else
+			for (r = 0; r < b->pend[i].rows; r++)
+				memcpy(d + r * b->pend[i].pitch, s + r * b->pend[i].pitch, b->pend[i].width);
+	}
 	b->npend = 0;
 	return e;
+}
+
+/* device-to-host copy of `rows` slots: the first `width` bytes of each, `pitch` apart on both sides (one flat copy
+ * when width == pitch) */
+static int d2h_slots(void *dst, const void *src, size_t width, size_t pitch, size_t rows, cudaStream_t s)
+{
+	if (!width || !rows)
+		return 0;
+	if (width == pitch)
+		return (int)cudaMemcpyAsync(dst, src, width * rows, cudaMemcpyDeviceToHost, s);
+	return (int)cudaMemcpy2DAsync(dst, pitch, src, pitch, width, rows, cudaMemcpyDeviceToHost, s);
 }
 
 /* optional page-locking of caller memory for the duration of a call ("host_register" knob) */
@@ -1259,13 +1284,14 @@ int csnappy_batch_compress_fragments_host(const void *h_in, uint64_t in_stride, 
 					  uint32_t *h_out_len, int workmem_bytes_power_of_two)
 {
 	int rc = 0, k, in_pg, out_pg;
-	size_t chunk, done;
+	size_t chunk, done, width;
 	struct ctx *c = NULL;
 	if (workmem_bytes_power_of_two < 9 || workmem_bytes_power_of_two > 16)
 		return set_err("workmem_bytes_power_of_two outside 9..16", 0);
 	if (uniform_in_len > CSB_FRAGMENT_MAX || in_stride < uniform_in_len ||
 	    out_stride < csnappy_max_compressed_length(uniform_in_len))
 		return set_err("bad block geometry", 0);
+	width = csnappy_max_compressed_length(uniform_in_len); /* bytes of a slot the kernel may write */
 	if (n_blocks == 0)
 		return 0;
 	if (!h_in || !h_out || !h_out_len)
@@ -1290,15 +1316,18 @@ int csnappy_batch_compress_fragments_host(const void *h_in, uint64_t in_stride, 
 	}
 	for (done = 0, k = 0; done < n_blocks; done += chunk, k = (k + 1) % PIPE) {
 		size_t nb = n_blocks - done < chunk ? n_blocks - done : chunk;
+		/* the last chunk ends with its last block: the caller's buffer need not extend to a whole stride */
+		const size_t in_bytes = done + nb == n_blocks ? (nb - 1) * in_stride + uniform_in_len : nb * in_stride;
 		struct slot *b = &c->sl[k];
 		struct csb_compress_args a;
 		const uint8_t *src = (const uint8_t *)h_in + done * in_stride;
 		TRY("copy-out of the slot's previous chunk", slot_drain(b));
 		if (in_pg) { /* pageable caller memory: through the slot's pinned staging (see par_memcpy) */
-			par_memcpy(b->h_in.p, src, nb * in_stride);
+			par_memcpy(b->h_in.p, src, in_bytes);
 			src = (const uint8_t *)b->h_in.p;
 		}
-		TRY("H2D", cudaMemcpyAsync(b->d_in.p, src, nb * in_stride, cudaMemcpyHostToDevice, b->s));
+		if (in_bytes)
+			TRY("H2D", cudaMemcpyAsync(b->d_in.p, src, in_bytes, cudaMemcpyHostToDevice, b->s));
 		fill_compress_args(&a);
 		a.in = (const uint8_t *)b->d_in.p;
 		a.in_stride = in_stride;
@@ -1313,11 +1342,10 @@ int csnappy_batch_compress_fragments_host(const void *h_in, uint64_t in_stride, 
 		if (out_pg) {
 			TRY("D2H data", cudaMemcpyAsync(b->h_out.p, b->d_slots.p, nb * out_stride, cudaMemcpyDeviceToHost, b->s));
 			TRY("D2H len", cudaMemcpyAsync(b->h_idx.p, b->d_len.p, nb * 4, cudaMemcpyDeviceToHost, b->s));
-			slot_owe(b, b->h_out.p, (uint8_t *)h_out + done * out_stride, nb * out_stride);
+			slot_owe2(b, b->h_out.p, (uint8_t *)h_out + done * out_stride, width, out_stride, nb);
 			slot_owe(b, b->h_idx.p, h_out_len + done, nb * 4);
 		} else {
-			TRY("D2H data", cudaMemcpyAsync((uint8_t *)h_out + done * out_stride, b->d_slots.p, nb * out_stride,
-							cudaMemcpyDeviceToHost, b->s));
+			TRY("D2H data", d2h_slots((uint8_t *)h_out + done * out_stride, b->d_slots.p, width, out_stride, nb, b->s));
 			TRY("D2H len", cudaMemcpyAsync(h_out_len + done, b->d_len.p, nb * 4, cudaMemcpyDeviceToHost, b->s));
 		}
 	}
@@ -1378,14 +1406,17 @@ int csnappy_batch_decompress_host(const void *h_in, uint64_t in_stride, const ui
 		struct slot *b = &c->sl[k];
 		uint32_t *d_ilen = (uint32_t *)b->d_res.p, *d_olen = d_ilen + chunk;
 		int32_t *d_st = (int32_t *)(d_olen + chunk);
+		/* the last chunk ends with its last block: the caller's buffer need not extend to a whole stride */
+		const size_t in_bytes = done + nb == n_blocks ? (nb - 1) * in_stride + h_in_len[n_blocks - 1] : nb * in_stride;
 		struct csb_decompress_args a;
 		const uint8_t *src = (const uint8_t *)h_in + done * in_stride;
 		TRY("copy-out of the slot's previous chunk", slot_drain(b));
 		if (in_pg) {
-			par_memcpy(b->h_in.p, src, nb * in_stride);
+			par_memcpy(b->h_in.p, src, in_bytes);
 			src = (const uint8_t *)b->h_in.p;
 		}
-		TRY("H2D", cudaMemcpyAsync(b->d_in.p, src, nb * in_stride, cudaMemcpyHostToDevice, b->s));
+		if (in_bytes)
+			TRY("H2D", cudaMemcpyAsync(b->d_in.p, src, in_bytes, cudaMemcpyHostToDevice, b->s));
 		TRY("H2D len", cudaMemcpyAsync(d_ilen, h_in_len + done, nb * 4, cudaMemcpyHostToDevice, b->s));
 		fill_decompress_args(&a);
 		a.in = (const uint8_t *)b->d_in.p;
@@ -1405,12 +1436,11 @@ int csnappy_batch_decompress_host(const void *h_in, uint64_t in_stride, const ui
 			TRY("D2H data", cudaMemcpyAsync(b->h_out.p, b->d_out.p, nb * out_stride, cudaMemcpyDeviceToHost, b->s));
 			TRY("D2H len", cudaMemcpyAsync(h_len, d_olen, nb * 4, cudaMemcpyDeviceToHost, b->s));
 			TRY("D2H status", cudaMemcpyAsync(h_st, d_st, nb * 4, cudaMemcpyDeviceToHost, b->s));
-			slot_owe(b, b->h_out.p, (uint8_t *)h_out + done * out_stride, nb * out_stride);
+			slot_owe2(b, b->h_out.p, (uint8_t *)h_out + done * out_stride, uniform_out_cap, out_stride, nb);
 			slot_owe(b, h_len, h_out_len + done, nb * 4);
 			slot_owe(b, h_st, h_status + done, nb * 4);
 		} else {
-			TRY("D2H data", cudaMemcpyAsync((uint8_t *)h_out + done * out_stride, b->d_out.p, nb * out_stride,
-							cudaMemcpyDeviceToHost, b->s));
+			TRY("D2H data", d2h_slots((uint8_t *)h_out + done * out_stride, b->d_out.p, uniform_out_cap, out_stride, nb, b->s));
 			TRY("D2H len", cudaMemcpyAsync(h_out_len + done, d_olen, nb * 4, cudaMemcpyDeviceToHost, b->s));
 			TRY("D2H status", cudaMemcpyAsync(h_status + done, d_st, nb * 4, cudaMemcpyDeviceToHost, b->s));
 		}

@@ -769,12 +769,11 @@ extern "C" int csb_launch_decompress(const struct csb_decompress_args *a, csb_st
 	// (32 KiB fragments: 116 vs 77 GB/s at 32 Ki, 300 vs 77 at 128 Ki) and ~150 Ki blocks against the staged path
 	// (mixed 4 KiB pages: 408 vs 417 GB/s at 128 Ki, 538 vs 430 at 256 Ki).  Needs 16-byte aligned output slots.
 	const bool lane_ok = ((reinterpret_cast<uintptr_t>(a->out) | a->out_stride) & 15u) == 0;
+	// stage_input 4 asks for it; slots it cannot write (the container reader's pages of any size, a caller's odd
+	// stride) take the routing below instead of failing the call
 	const uint32_t lane_min = (uint32_t)di.sm_count * (unstaged ? 160u : 1100u);
-	if (a->stage_input == 4 || (a->stage_input == 0 && lane_ok && a->n_blocks >= lane_min)) {
-		if (!lane_ok)
-			return (int)cudaErrorMisalignedAddress;
+	if (lane_ok && (a->stage_input == 4 || (a->stage_input == 0 && a->n_blocks >= lane_min)))
 		return csb_launch_decompress_lane(a, s);
-	}
 	if (unstaged) {
 		// too few blocks fit shared memory for their chains to hide each other: global path, one group per warp slot
 		p.in_area = p.out_area = 0;

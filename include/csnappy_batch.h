@@ -125,7 +125,16 @@ int csnappy_batch_pack(const void *d_slots, uint64_t slot_stride,
  * Host-buffer variants: same semantics, HOST pointers, synchronous.  Pages are
  * streamed through the device in chunks on several CUDA streams so that H2D,
  * kernels and D2H overlap.  These are what a zram / block_compressor style
- * caller with host memory uses, and what bench.py times as "e2e".
+ * caller with host memory uses.
+ *
+ * Bytes of the caller's memory these calls touch: block i is read from
+ * h_in + i * in_stride for its own length only (uniform_in_len / h_in_len[i]),
+ * so h_in needs (n_blocks - 1) * in_stride + the last block's length bytes.
+ * Of output slot i only the first csnappy_max_compressed_length(uniform_in_len)
+ * (compress) or uniform_out_cap (decompress) bytes are written: whatever the
+ * caller keeps in the rest of each slot, and after the last slot's bound,
+ * stays as it was.  Inside that bound, bytes past h_out_len[i] (and all of a
+ * slot whose block failed to decode) have unspecified values.
  */
 int csnappy_batch_compress_fragments_host(const void *h_in, uint64_t in_stride,
 					  uint32_t uniform_in_len, uint32_t n_blocks,
@@ -154,6 +163,13 @@ int csnappy_batch_decompress_host(const void *h_in, uint64_t in_stride,
  * csnappy_bc_decompress_host  out_capacity >= nr_pages * page_size (CSNAPPY_E_OUTPUT_INSUF else);
  *                             returns 0 or the code of the first failing page (its index goes to
  *                             *failed_page when given); *out_length = bytes produced.
+ *                             The index is scanned first: the first entry above
+ *                             csnappy_max_compressed_length(page_size), or whose payload runs past
+ *                             container_length, fails its page with CSNAPPY_E_DATA_MALFORMED and ends
+ *                             the decodable prefix.  Every page of that prefix is decoded, those after
+ *                             a failing page too; *out_length sums what the prefix's successful pages
+ *                             produced.  Page i goes to h_out + i * page_size; the bytes of a failed
+ *                             page are unspecified, pages past the prefix are not written.
  */
 uint64_t csnappy_bc_max_container_length(uint64_t input_length, uint32_t page_size);
 int csnappy_bc_compress_host(const void *h_in, uint64_t input_length, uint32_t page_size,
@@ -194,7 +210,8 @@ uint64_t csnappy_b200_kernel_launches(void); /* kernels launched by this library
  *                             groups only; the default for large batches of fragments above ~14 KB)
  *   "decompress_stage_input"  1: always stage blocks in shared memory; 2: stage only the output and read the
  *                             compressed block through L1; 3: decode against global memory, a warp per block;
- *                             4: one lane per block (the default for very large batches)
+ *                             4: one lane per block (the default for very large batches; it needs 16-byte
+ *                             aligned output slots, other layouts keep the default routing)
  *   "decompress_lane_warps"   lane-per-block decoder: warps of 32 blocks in flight per SM (default 32)
  *   "decompress_smem_kb"      shared memory per SM in mode 2
  *   "ctas_per_sm"             resident CTAs per SM of the warp-per-block kernels

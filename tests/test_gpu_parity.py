@@ -14,6 +14,7 @@ import pytest
 
 import oracle
 from cases import fuzz_pages, synth_cases
+from containers import ref_container
 
 pytestmark = pytest.mark.gpu
 
@@ -300,20 +301,6 @@ def test_c_caller_through_the_plain_c_abi(cs, urls, urls_snappy, tmp_path):
 
 
 # --------------------------------------------------------------------------- block_compressor container
-def _ref_container(chk, data: bytes, page: int, wm: int) -> bytes:
-    """block_compressor.c:275-345 restated with the oracle as the page compressor."""
-    nr = (len(data) + page - 1) // page
-    idx, payload = [], []
-    for i in range(nr):
-        p = data[i * page:(i + 1) * page]
-        c = chk.compress_fragment(p, wm)
-        if len(c) >= len(p):
-            c = p
-        idx.append(len(c))
-        payload.append(c)
-    return struct.pack("<I", nr) + b"".join(struct.pack("<I", x) for x in idx) + b"".join(payload)
-
-
 @pytest.mark.parametrize("page,wm", [(4096, 13), (1024, 11), (32768, 15)])
 def test_bc_container_matches_reference_writer_and_round_trips(cs, chk, urls, page, wm):
     rng = np.random.default_rng(21)
@@ -322,7 +309,7 @@ def test_bc_container_matches_reference_writer_and_round_trips(cs, chk, urls, pa
     h_in = np.frombuffer(data, dtype=np.uint8).copy()
     cont = np.zeros(cs.api.bc_max_container_length(len(data), page), dtype=np.uint8)
     clen = cs.api.bc_compress_host(h_in, len(data), cont, wm, page)
-    ref = _ref_container(chk, data, page, wm)
+    ref = ref_container(chk, data, page, wm)
     assert clen == len(ref) and cont[:clen].tobytes() == ref
     nr = (len(data) + page - 1) // page
     out = np.zeros(nr * page, dtype=np.uint8)

@@ -3,7 +3,9 @@
 compressed bytes and decoder results compared with the unmodified reference (oracle/_ref).  The compress leg
 also gets blocks built to drive the parse through the kernel's rare paths (tests/compress_cases.py: hash-slot
 sharing in stride-1 and strided windows, in-window copies, the scan end, length and offset boundaries); the decode
-leg gets random streams of every tag form (tests/streams.py), which the compressor never writes.
+leg gets random streams of every tag form (tests/streams.py), which the compressor never writes.  The container leg
+writes a page container of random page size and length, corrupts its index and payload at random and compares the
+reader with the restated reader (tests/containers.py).
 
     python tools/fuzz_gpu.py [seconds] [seed]
 """
@@ -18,6 +20,7 @@ sys.path.insert(0, "tests")
 import csnappy_b200 as cs
 import oracle
 import compress_cases
+import containers
 from cases import fuzz_pages
 from streams import random_stream
 
@@ -26,7 +29,7 @@ seed = int(sys.argv[2]) if len(sys.argv) > 2 else 20261017
 chk = oracle.best()
 rng = np.random.default_rng(seed)
 t0 = time.time()
-rounds = blocks = streams = 0
+rounds = blocks = streams = pages_read = 0
 while time.time() - t0 < budget:
     size = int(rng.choice([17, 64, 300, 1000, 4096, 4096, 4096, 5000, 16384, 32768]))
     wm = int(rng.integers(9, 17))
@@ -101,10 +104,33 @@ while time.time() - t0 < budget:
         if rc == 0:
             assert bl[i] == len(exp) and bo[i * max(ocap, 16): i * max(ocap, 16) + bl[i]].tobytes() == exp, ("bytes", size, lanes, i)
     streams += n_dec
+    # container: random page size and length, the index and payloads corrupted at random, against the restated reader
+    page = int(rng.choice([1, 17, 1000, 4095, 4096, 4097, 20000, 32768]))
+    data = containers.mixed_bytes(int(rng.integers(1 << 30)), int(rng.integers(1, 600 * page + 2)), scale=max(page, 64))
+    cont = np.zeros(cs.api.bc_max_container_length(len(data), page), dtype=np.uint8)
+    clen = cs.api.bc_compress_host(np.frombuffer(data, dtype=np.uint8), len(data), cont, wm, page)
+    assert cont[:clen].tobytes() == containers.ref_container(chk, data, page, wm), ("container", page, len(data), wm)
+    broken = bytearray(cont[:clen].tobytes())
+    nr = (len(data) + page - 1) // page
+    for _ in range(int(rng.integers(0, 4))):
+        i = int(rng.integers(0, nr))
+        broken[4 + 4 * i: 8 + 4 * i] = int(rng.choice([0, page - 1, page, page + 1, 32 + page + page // 6 + 1,
+                                                        int(rng.integers(0, 2 * page + 40))])).to_bytes(4, "little")
+    for _ in range(int(rng.integers(0, 4))):
+        broken[int(rng.integers(4 + 4 * nr, len(broken) + 1)) - 1] ^= int(rng.integers(1, 256))
+    if rng.random() < 0.2:
+        broken = broken[: int(rng.integers(4, len(broken) + 1))]
+    want = containers.read_container(bytes(broken), page, nr * page)
+    out = np.zeros(nr * page, dtype=np.uint8)
+    rc, olen, bad = cs.api.bc_decompress_host(np.frombuffer(bytes(broken), dtype=np.uint8), len(broken), out, page)
+    assert (rc, olen, bad) == want.key(), ("container read", page, len(data), want.key(), (rc, olen, bad))
+    for i, b in want.pages.items():
+        assert out[i * page: i * page + len(b)].tobytes() == b, ("container page", page, i)
+    pages_read += nr
     rounds += 1
 cs.set_tuning("compress_lanes", 0)
 cs.set_tuning("decompress_lanes", 0)
 cs.set_tuning("compress_stage_input", 0)
 cs.set_tuning("decompress_stage_input", 0)
-print(f"fuzz ok: {rounds} rounds, {blocks} blocks compressed byte-identically, {streams} streams decoded with identical results "
-      f"in {time.time() - t0:.0f} s")
+print(f"fuzz ok: {rounds} rounds, {blocks} blocks compressed byte-identically, {streams} streams decoded with identical results, "
+      f"{pages_read} container pages written and read as restated in {time.time() - t0:.0f} s")
