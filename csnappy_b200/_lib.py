@@ -41,6 +41,14 @@ def _declare(L):
         "csnappy_bc_decompress_host_multi": (i, [vp, u64, u32, vp, u64, C.POINTER(C.c_uint64), _u32p, vp, i]),
         "csnappy_stream_decompress_workspace": (u64, [u32, u32]),
         "csnappy_stream_decompress": (i, [vp, u32, vp, u32, vp, vp, vp, u64, vp]),
+        "csnappy_framed_max_length": (u64, [u64]),
+        "csnappy_framed_compress_workspace": (u64, [u64]),
+        "csnappy_framed_compress": (i, [vp, u64, vp, u64, vp, i, vp, u64, vp]),
+        "csnappy_framed_decompress_workspace": (u64, [u64]),
+        "csnappy_framed_decompress": (i, [vp, u64, vp, u64, vp, vp, vp, vp, u64, vp]),
+        "csnappy_framed_compress_host": (i, [vp, u64, vp, u64, C.POINTER(C.c_uint64), i]),
+        "csnappy_framed_decompress_host": (i, [vp, u64, vp, u64, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
+        "csnappy_framed_crc32c": (i, [vp, u64, vp, vp]),
         "csnappy_b200_device_count": (i, []),
         "csnappy_b200_device_ok": (i, []),
         "csnappy_b200_last_error": (C.c_char_p, []),

@@ -12,6 +12,9 @@ Device-resident batches (torch CUDA tensors, asynchronous on the current stream)
     batch_compress_fragments, batch_decompress, batch_pack
 Host-buffer batches (numpy / pinned torch tensors, synchronous, pipelined H2D/D2H):
     batch_compress_fragments_host, batch_decompress_host
+Snappy framing format (64 KiB chunks with masked CRC-32C):
+    framed_compress, framed_decompress (host bytes); framed_compress_device, framed_decompress_device,
+    framed_crc32c_device (CUDA tensors, current stream)
 """
 from __future__ import annotations
 
@@ -308,3 +311,96 @@ def kernel_launches() -> int:
 
 def device_ok() -> bool:
     return bool(lib().csnappy_b200_device_ok())
+
+
+# ----------------------------------------------------------------------------- Snappy framing format
+CSNAPPY_E_CHECKSUM = -102
+FRAMED_CHUNK = 65536
+
+
+def framed_max_length(input_length: int) -> int:
+    """Exact bound of a framed stream of input_length bytes: 10 + 8 * ceil(n / 65536) + n."""
+    return lib().csnappy_framed_max_length(input_length)
+
+
+def framed_compress(data, wm: int = CSNAPPY_WORKMEM_BYTES_POWER_OF_TWO) -> bytes:
+    """Host bytes -> one framed stream (stream identifier, 64 KiB chunks with masked CRC-32C)."""
+    n = len(data)
+    src = _in_buf(data)
+    out = np.empty(framed_max_length(n), dtype=np.uint8)
+    olen = C.c_uint64(0)
+    rc = lib().csnappy_framed_compress_host(src.ctypes.data, n, out.ctypes.data, out.nbytes, C.byref(olen), wm)
+    _check(rc, "csnappy_framed_compress_host")
+    return out[: olen.value].tobytes()
+
+
+def framed_decompress(data, out_capacity: int):
+    """Host bytes of a framed stream -> (rc, the valid prefix of the output, failed_offset or None).
+    rc: 0, CSNAPPY_E_OUTPUT_INSUF, CSNAPPY_E_DATA_MALFORMED or CSNAPPY_E_CHECKSUM; failed_offset is the header
+    position of the failing chunk."""
+    src = _in_buf(data)
+    out = np.empty(max(out_capacity, 1), dtype=np.uint8)
+    olen = C.c_uint64(0)
+    bad = C.c_uint64(0)
+    rc = lib().csnappy_framed_decompress_host(src.ctypes.data, len(data), out.ctypes.data, out_capacity,
+                                              C.byref(olen), C.byref(bad))
+    if rc in (CSNAPPY_E_DEVICE, CSNAPPY_E_BAD_ARG):
+        _check(rc, "csnappy_framed_decompress_host")
+    return rc, out[: olen.value].tobytes(), (bad.value if rc != 0 else None)
+
+
+def framed_compress_device(d_in, input_length: int | None = None, wm: int = CSNAPPY_WORKMEM_BYTES_POWER_OF_TWO, *,
+                           out=None, out_length=None, workspace=None):
+    """Device-resident framed compress of a uint8 CUDA tensor, asynchronous on the current stream.
+    Returns (out uint8 [framed_max_length(n)], out_length int64 [1]) CUDA tensors."""
+    import torch
+
+    n = d_in.numel() if input_length is None else input_length
+    cap = framed_max_length(n)
+    if out is None:
+        out = torch.empty(cap, dtype=torch.uint8, device=d_in.device)
+    if out_length is None:
+        out_length = torch.empty(1, dtype=torch.int64, device=d_in.device)
+    ws_bytes = lib().csnappy_framed_compress_workspace(n)
+    if workspace is None:
+        workspace = torch.empty(ws_bytes, dtype=torch.uint8, device=d_in.device)
+    rc = lib().csnappy_framed_compress(_ptr(d_in), n, _ptr(out), out.numel(), _ptr(out_length), wm, _ptr(workspace),
+                                       workspace.numel(), _stream_ptr())
+    _check(rc, "csnappy_framed_compress")
+    return out, out_length  # the workspace is freed in stream order: the caching allocator reuses it after this work
+
+
+def framed_decompress_device(d_src, src_length: int | None = None, out_capacity: int = 0, *, out=None, result=None,
+                             workspace=None):
+    """Device-resident framed decompress, on the current stream (the call waits for the chunk walk, then enqueues
+    decoding and verification).  Returns (out uint8 [out_capacity], result int64 [3] = [out_length, rc,
+    failed_offset]) CUDA tensors; result[2] is written only when rc != 0."""
+    import torch
+
+    n = d_src.numel() if src_length is None else src_length
+    if out is None:
+        out = torch.empty(max(out_capacity, 1), dtype=torch.uint8, device=d_src.device)
+    if result is None:
+        result = torch.full((3,), -1, dtype=torch.int64, device=d_src.device)
+    ws_bytes = lib().csnappy_framed_decompress_workspace(n)
+    if workspace is None:
+        workspace = torch.empty(ws_bytes, dtype=torch.uint8, device=d_src.device)
+    status = torch.zeros(1, dtype=torch.int32, device=d_src.device)
+    rc = lib().csnappy_framed_decompress(_ptr(d_src), n, _ptr(out), out_capacity, result.data_ptr(), status.data_ptr(),
+                                         result.data_ptr() + 16, _ptr(workspace), workspace.numel(), _stream_ptr())
+    _check(rc, "csnappy_framed_decompress")
+    result[1:2].copy_(status)
+    return out, result
+
+
+def framed_crc32c_device(d_in, length: int | None = None, *, crc=None):
+    """Masked CRC-32C of each 64 KiB chunk of a uint8 CUDA tensor -> int32 CUDA tensor (as uint32 bits)."""
+    import torch
+
+    n = d_in.numel() if length is None else length
+    k = -(-n // FRAMED_CHUNK)
+    if crc is None:
+        crc = torch.empty(max(k, 1), dtype=torch.int32, device=d_in.device)
+    rc = lib().csnappy_framed_crc32c(_ptr(d_in), n, _ptr(crc), _stream_ptr())
+    _check(rc, "csnappy_framed_crc32c")
+    return crc

@@ -22,7 +22,8 @@ LIB = os.path.join(HERE, "libcsnappy_b200" + ("_" + TAG if TAG else "") + ".so")
 CUDA_HOME = os.environ.get("CUDA_HOME", "/usr/local/cuda")
 NVCC = shutil.which("nvcc") or os.path.join(CUDA_HOME, "bin", "nvcc")
 
-CU = ["compress_kernel.cu", "decompress_kernel.cu", "decompress_lane_kernel.cu", "stream_kernel.cu", "pack_kernel.cu"]
+CU = ["compress_kernel.cu", "decompress_kernel.cu", "decompress_lane_kernel.cu", "stream_kernel.cu", "pack_kernel.cu",
+      "framed_kernel.cu"]
 C = ["csnappy_shim.c"]
 HEADERS = [os.path.join(CSRC, h) for h in ("kernels.h", "device_common.cuh")] + [
     os.path.join(HERE, "..", "include", h) for h in ("csnappy.h", "csnappy_batch.h")

@@ -1813,3 +1813,273 @@ int csnappy_bc_decompress_host_multi(const void *h_container, uint64_t container
 		return G;
 	return bc_decompress(h_container, container_length, page_size, h_out, out_capacity, out_length, failed_page, list, G);
 }
+
+/* ---- Snappy framing format (include/csnappy_batch.h csnappy_framed_*; kernels in framed_kernel.cu) ------------------
+ * Writer: ONE compress launch over the whole input as 32 KiB fragments (only the global last fragment is short, and it
+ * gets csnappy_compress()'s short-chunk table rule), so fragments 2k and 2k+1 behind a varint are exactly
+ * csnappy_compress(chunk k).  Then one warp per chunk computes its masked CRC-32C and record size, a scan places the
+ * records, and one warp per chunk writes header, CRC and payload.
+ * Reader: one thread walks the chunk headers (a dependent chain) into a table of data chunks; the host reads the
+ * counts back to size the launches; the batched decoder writes every compressed chunk straight to its output offset;
+ * one warp per data chunk copies stored chunks and checks lengths and CRCs; one thread writes the result.           */
+#define FRAMED_CHUNK ((uint64_t)CSB_FRAMED_CHUNK)
+#define FRAMED_IDENT 10u
+
+static uint64_t chunks_of(uint64_t n) { return (n + FRAMED_CHUNK - 1) / FRAMED_CHUNK; }
+
+uint64_t csnappy_framed_max_length(uint64_t input_length)
+{
+	return FRAMED_IDENT + 8 * chunks_of(input_length) + input_length;
+}
+
+/* workspace of the writer: fragment slots | fragment sizes | crc | record sizes | record offsets | counter */
+static uint64_t framed_compress_layout(uint64_t n, uint64_t *o_flen, uint64_t *o_crc, uint64_t *o_rec, uint64_t *o_off,
+				       uint64_t *o_ctr)
+{
+	const uint64_t F = (n + CSB_FRAGMENT_MAX - 1) / CSB_FRAGMENT_MAX, K = chunks_of(n);
+	uint64_t p = al256(F * SLOT_STRIDE_32K);
+	*o_flen = p;
+	p = al256(p + F * 4);
+	*o_crc = p;
+	p = al256(p + K * 4);
+	*o_rec = p;
+	p = al256(p + K * 4);
+	*o_off = p;
+	p = al256(p + (K + 1) * 8);
+	*o_ctr = p;
+	return p + 256;
+}
+
+uint64_t csnappy_framed_compress_workspace(uint64_t input_length)
+{
+	uint64_t a, b, c, d, e;
+	return framed_compress_layout(input_length, &a, &b, &c, &d, &e);
+}
+
+/* the longest input: 2^32 - 1 fragments of 32 KiB for the compress launch */
+#define FRAMED_MAX_INPUT (((uint64_t)0xffffffffu - 1) * CSB_FRAGMENT_MAX)
+
+int csnappy_framed_compress(const void *d_in, uint64_t input_length, void *d_out, uint64_t out_capacity,
+			    uint64_t *d_out_length, int workmem_bytes_power_of_two, void *d_workspace, uint64_t workspace_bytes,
+			    void *stream)
+{
+	uint64_t o_flen, o_crc, o_rec, o_off, o_ctr, need;
+	const uint64_t F = (input_length + CSB_FRAGMENT_MAX - 1) / CSB_FRAGMENT_MAX;
+	uint8_t *ws = (uint8_t *)d_workspace;
+	csb_stream_t s = (csb_stream_t)stream;
+	struct csb_compress_args a;
+	int e;
+	if (workmem_bytes_power_of_two < 9 || workmem_bytes_power_of_two > 16)
+		return set_err("workmem_bytes_power_of_two outside 9..16", 0);
+	if (input_length > FRAMED_MAX_INPUT)
+		return set_err("input longer than (2^32 - 2) * 32768 bytes", 0);
+	if ((input_length && !d_in) || !d_out || !d_out_length || !d_workspace)
+		return set_err("null buffer", 0);
+	if (out_capacity < csnappy_framed_max_length(input_length))
+		return set_err("out_capacity smaller than csnappy_framed_max_length()", 0);
+	need = framed_compress_layout(input_length, &o_flen, &o_crc, &o_rec, &o_off, &o_ctr);
+	if (workspace_bytes < need)
+		return set_err("workspace smaller than csnappy_framed_compress_workspace()", 0);
+	if (F) {
+		fill_compress_args(&a);
+		a.in = (const uint8_t *)d_in;
+		a.in_stride = CSB_FRAGMENT_MAX;
+		a.uniform_len = CSB_FRAGMENT_MAX;
+		a.total_len = input_length;
+		a.n_blocks = (uint32_t)F;
+		a.out = ws;
+		a.out_stride = SLOT_STRIDE_32K;
+		a.out_len = (uint32_t *)(ws + o_flen);
+		a.wm = workmem_bytes_power_of_two;
+		a.flags = CSNAPPY_BATCH_SHRINK_TABLE;
+		a.counter = (uint32_t *)(ws + o_ctr);
+		if ((e = csb_launch_compress(&a, s)))
+			return set_err("compress launch", e);
+		if ((e = csb_launch_framed_crc((const uint8_t *)d_in, input_length, (uint32_t *)(ws + o_crc),
+					       (const uint32_t *)(ws + o_flen), (uint32_t)F, (uint32_t *)(ws + o_rec), s)))
+			return set_err("crc launch", e);
+	}
+	if ((e = csb_launch_scan((const uint32_t *)(ws + o_rec), (uint32_t)chunks_of(input_length), (uint64_t *)(ws + o_off), s)))
+		return set_err("scan launch", e);
+	e = csb_launch_framed_write((const uint8_t *)d_in, input_length, ws, SLOT_STRIDE_32K, (const uint32_t *)(ws + o_flen),
+				    (uint32_t)F, (const uint32_t *)(ws + o_crc), (const uint32_t *)(ws + o_rec),
+				    (const uint64_t *)(ws + o_off), (uint8_t *)d_out, d_out_length, s);
+	return e ? set_err("framed write launch", e) : 0;
+}
+
+int csnappy_framed_crc32c(const void *d_in, uint64_t length, uint32_t *d_crc, void *stream)
+{
+	int e;
+	if (length > FRAMED_MAX_INPUT)
+		return set_err("input longer than (2^32 - 2) * 32768 bytes", 0);
+	if (length && (!d_in || !d_crc))
+		return set_err("null buffer", 0);
+	e = csb_launch_framed_crc((const uint8_t *)d_in, length, d_crc, NULL, 0, NULL, (csb_stream_t)stream);
+	return e ? set_err("crc launch", e) : 0;
+}
+
+/* Reader workspace: result words, then the tables of csb_framed_table for at most src_length / 8 + 1 data chunks (a
+ * data chunk takes at least 8 bytes of the stream), then the decoder's block counter. */
+#define FRAMED_MAX_SRC ((uint64_t)0xfffffffeu * 8)
+
+static uint64_t framed_decompress_layout(uint64_t src_length, struct csb_framed_table *t, uint8_t *ws, uint32_t **ctr)
+{
+	const uint64_t D = src_length / 8 + 1;
+	uint64_t p = 0;
+#define FRAMED_TAB(field, type, per)                              \
+	do {                                                      \
+		if (t)                                            \
+			t->field = (type *)(ws + p);              \
+		p = al256(p + (per));                             \
+	} while (0)
+	FRAMED_TAB(res, struct csb_framed_result, sizeof(struct csb_framed_result));
+	FRAMED_TAB(pos, uint64_t, D * 8);
+	FRAMED_TAB(out_off, uint64_t, D * 8);
+	FRAMED_TAB(out_len, uint32_t, D * 4);
+	FRAMED_TAB(crc, uint32_t, D * 4);
+	FRAMED_TAB(cidx, uint32_t, D * 4);
+	FRAMED_TAB(c_pos, uint64_t, D * 8);
+	FRAMED_TAB(c_out_off, uint64_t, D * 8);
+	FRAMED_TAB(c_len, uint32_t, D * 4);
+	FRAMED_TAB(c_produced, uint32_t, D * 4);
+	FRAMED_TAB(c_status, int32_t, D * 4);
+#undef FRAMED_TAB
+	if (ctr)
+		*ctr = (uint32_t *)(ws + p);
+	return p + 256;
+}
+
+uint64_t csnappy_framed_decompress_workspace(uint64_t src_length)
+{
+	return framed_decompress_layout(src_length, NULL, NULL, NULL);
+}
+
+int csnappy_framed_decompress(const void *d_src, uint64_t src_length, void *d_dst, uint64_t out_capacity,
+			      uint64_t *d_out_length, int32_t *d_status, uint64_t *d_failed_offset, void *d_workspace,
+			      uint64_t workspace_bytes, void *stream)
+{
+	struct csb_framed_table t;
+	struct csb_framed_result r;
+	struct csb_decompress_args a;
+	uint32_t *ctr = NULL;
+	cudaStream_t s = (cudaStream_t)stream;
+	const uint8_t *src = (const uint8_t *)d_src;
+	int e;
+	if (src_length > FRAMED_MAX_SRC)
+		return set_err("src_length above 2^35 bytes", 0);
+	if ((src_length && !d_src) || (out_capacity && !d_dst) || !d_out_length || !d_status || !d_workspace)
+		return set_err("null buffer", 0);
+	if (workspace_bytes < csnappy_framed_decompress_workspace(src_length))
+		return set_err("workspace smaller than csnappy_framed_decompress_workspace()", 0);
+	framed_decompress_layout(src_length, &t, (uint8_t *)d_workspace, &ctr);
+	if ((e = csb_launch_framed_walk(src, src_length, out_capacity, &t, (csb_stream_t)s)))
+		return set_err("framed walk launch", e);
+	/* the only synchronisation: the chunk counts size the launches below */
+	if ((e = (int)cudaMemcpyAsync(&r, t.res, sizeof(r), cudaMemcpyDeviceToHost, s)) || (e = (int)cudaStreamSynchronize(s)))
+		return set_err("D2H chunk counts", e);
+	if (r.n_comp) {
+		fill_decompress_args(&a);
+		a.in = src + 8; /* block j = the body behind chunk j's header and CRC */
+		a.in_off = t.c_pos;
+		a.in_len = t.c_len;
+		a.n_blocks = r.n_comp;
+		a.out = (uint8_t *)d_dst;
+		a.out_off = t.c_out_off;
+		a.uniform_cap = CSB_FRAMED_CHUNK; /* WITH_HEADER: the capacity becomes the varint's value, <= 65536 */
+		a.out_len = t.c_produced;
+		a.status = t.c_status;
+		a.flags = CSNAPPY_BATCH_WITH_HEADER;
+		a.counter = ctr;
+		if ((e = csb_launch_decompress(&a, (csb_stream_t)s)))
+			return set_err("decompress launch", e);
+	}
+	e = csb_launch_framed_verify(src, (uint8_t *)d_dst, r.n_data, &t, d_out_length, d_status, d_failed_offset,
+				     (csb_stream_t)s);
+	return e ? set_err("framed verify launch", e) : 0;
+}
+
+/* Host buffers: the whole input and output staged through one pooled context. */
+int csnappy_framed_compress_host(const void *h_in, uint64_t input_length, void *h_out, uint64_t out_capacity,
+				 uint64_t *out_length, int workmem_bytes_power_of_two)
+{
+	int rc = 0;
+	struct ctx *c = NULL;
+	struct slot *sl;
+	uint64_t max_len = csnappy_framed_max_length(input_length), olen = 0;
+	if (workmem_bytes_power_of_two < 9 || workmem_bytes_power_of_two > 16)
+		return set_err("workmem_bytes_power_of_two outside 9..16", 0);
+	if (input_length > FRAMED_MAX_INPUT)
+		return set_err("input longer than (2^32 - 2) * 32768 bytes", 0);
+	if ((input_length && !h_in) || !h_out || !out_length)
+		return set_err("null buffer", 0);
+	if (out_capacity < max_len)
+		return set_err("out_capacity smaller than csnappy_framed_max_length()", 0);
+	TRY("context", ctx_acquire(&c));
+	sl = &c->sl[0];
+	TRY("cudaMalloc(in)", grow_dev_retry(&sl->d_in, (size_t)input_length + 64));
+	TRY("cudaMalloc(out)", grow_dev_retry(&sl->d_out, (size_t)max_len + 64));
+	TRY("cudaMalloc(res)", grow_dev_retry(&sl->d_res, 64));
+	TRY("cudaMalloc(workspace)", grow_dev_retry(&c->d_aux, (size_t)csnappy_framed_compress_workspace(input_length)));
+	if (input_length)
+		TRY("H2D", cudaMemcpyAsync(sl->d_in.p, h_in, (size_t)input_length, cudaMemcpyHostToDevice, sl->s));
+	rc = csnappy_framed_compress(sl->d_in.p, input_length, sl->d_out.p, max_len, (uint64_t *)sl->d_res.p,
+				     workmem_bytes_power_of_two, c->d_aux.p, c->d_aux.cap, sl->s);
+	if (rc)
+		goto out;
+	TRY("D2H length", cudaMemcpyAsync(&olen, sl->d_res.p, 8, cudaMemcpyDeviceToHost, sl->s));
+	TRY("sync", cudaStreamSynchronize(sl->s));
+	TRY("D2H data", cudaMemcpyAsync(h_out, sl->d_out.p, (size_t)olen, cudaMemcpyDeviceToHost, sl->s));
+	TRY("sync", cudaStreamSynchronize(sl->s));
+	*out_length = olen;
+out:
+	ctx_release(c);
+	return rc;
+}
+
+int csnappy_framed_decompress_host(const void *h_src, uint64_t src_length, void *h_dst, uint64_t out_capacity,
+				   uint64_t *out_length, uint64_t *failed_offset)
+{
+	int rc = 0;
+	struct ctx *c = NULL;
+	struct slot *sl;
+	/* no stream can produce more than 65536 bytes per 9 of its bytes: a larger capacity needs no device memory */
+	const uint64_t most = (src_length / 9 + 1) * FRAMED_CHUNK, cap = out_capacity < most ? out_capacity : most;
+	struct {
+		uint64_t out_length;
+		uint64_t failed_offset;
+		int32_t status;
+		int32_t pad;
+	} res = {0, 0, 0, 0};
+	if (src_length > FRAMED_MAX_SRC)
+		return set_err("src_length above 2^35 bytes", 0);
+	if ((src_length && !h_src) || (out_capacity && !h_dst) || !out_length)
+		return set_err("null buffer", 0);
+	TRY("context", ctx_acquire(&c));
+	sl = &c->sl[0];
+	TRY("cudaMalloc(in)", grow_dev_retry(&sl->d_in, (size_t)src_length + 64));
+	TRY("cudaMalloc(out)", grow_dev_retry(&sl->d_out, (size_t)cap + 64));
+	TRY("cudaMalloc(res)", grow_dev_retry(&sl->d_res, 64));
+	TRY("cudaMalloc(workspace)", grow_dev_retry(&c->d_aux, (size_t)csnappy_framed_decompress_workspace(src_length)));
+	if (src_length)
+		TRY("H2D", cudaMemcpyAsync(sl->d_in.p, h_src, (size_t)src_length, cudaMemcpyHostToDevice, sl->s));
+	{
+		uint8_t *d_res = (uint8_t *)sl->d_res.p;
+		rc = csnappy_framed_decompress(sl->d_in.p, src_length, sl->d_out.p, cap, (uint64_t *)d_res, (int32_t *)(d_res + 16),
+					       (uint64_t *)(d_res + 8), c->d_aux.p, c->d_aux.cap, sl->s);
+		if (rc)
+			goto out;
+	}
+	TRY("D2H result", cudaMemcpyAsync(&res, sl->d_res.p, sizeof(res), cudaMemcpyDeviceToHost, sl->s));
+	TRY("sync", cudaStreamSynchronize(sl->s));
+	if (res.out_length) {
+		TRY("D2H data", cudaMemcpyAsync(h_dst, sl->d_out.p, (size_t)res.out_length, cudaMemcpyDeviceToHost, sl->s));
+		TRY("sync", cudaStreamSynchronize(sl->s));
+	}
+	*out_length = res.out_length;
+	rc = res.status;
+	if (rc && failed_offset)
+		*failed_offset = res.failed_offset;
+out:
+	ctx_release(c);
+	return rc;
+}

@@ -576,7 +576,7 @@ __global__ void __launch_bounds__(kMaxThreadsD, 1) decompress_kernel(const Decom
 			const uint8_t *src = a.in + (a.in_off ? a.in_off[blk] : (uint64_t)blk * a.in_stride);
 			uint32_t ilen = a.in_len[blk];
 			uint32_t cap = a.out_cap ? a.out_cap[blk] : a.uniform_cap;
-			dst = a.out + (uint64_t)blk * a.out_stride;
+			dst = a.out + (a.out_off ? a.out_off[blk] : (uint64_t)blk * a.out_stride);
 			int rc = E_OK;
 			if (a.flags & 2u) {  // varint32 length prefix, csnappy_decompress.c:45-71, 404-409
 				uint32_t shift = 0, used = 0, value = 0;
@@ -768,7 +768,7 @@ extern "C" int csb_launch_decompress(const struct csb_decompress_args *a, csb_st
 	// (1280 per SM): measured crossovers on a B200 are ~24 Ki blocks against the warp-per-block global path
 	// (32 KiB fragments: 116 vs 77 GB/s at 32 Ki, 300 vs 77 at 128 Ki) and ~150 Ki blocks against the staged path
 	// (mixed 4 KiB pages: 408 vs 417 GB/s at 128 Ki, 538 vs 430 at 256 Ki).  Needs 16-byte aligned output slots.
-	const bool lane_ok = ((reinterpret_cast<uintptr_t>(a->out) | a->out_stride) & 15u) == 0;
+	const bool lane_ok = !a->out_off && ((reinterpret_cast<uintptr_t>(a->out) | a->out_stride) & 15u) == 0;
 	// stage_input 4 asks for it; slots it cannot write (the container reader's pages of any size, a caller's odd
 	// stride) take the routing below instead of failing the call
 	const uint32_t lane_min = (uint32_t)di.sm_count * (unstaged ? 160u : 1100u);

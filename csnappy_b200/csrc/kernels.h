@@ -45,6 +45,8 @@ struct csb_decompress_args {
 	uint32_t n_blocks;
 	uint8_t *out;
 	uint64_t out_stride;
+	const uint64_t *out_off; /* NULL => i * out_stride; set: block i's output at out + out_off[i] (the lane-per-block
+				    decoder, which needs 16-byte aligned strided slots, is then not selected) */
 	const uint32_t *out_cap; /* NULL => uniform_cap */
 	uint32_t uniform_cap;
 	uint32_t *out_len;
@@ -80,6 +82,32 @@ size_t csb_stream_aux_bytes(uint32_t src_len, uint32_t cap, int which);
 int csb_launch_decompress_stream(const uint8_t *d_in, uint32_t src_len, uint8_t *d_out, uint32_t cap, uint32_t *d_out_len,
 				 int32_t *d_status, void *d_aux_in, void *d_aux_out, csb_stream_t s);
 uint64_t csb_launch_count(void);
+
+/* Snappy framing format (framed_kernel.cu) */
+#define CSB_FRAMED_CHUNK 65536u
+struct csb_framed_result {	/* device word block of one framed read */
+	uint32_t n_data, n_comp; /* data chunks / compressed chunks the walk recorded */
+	uint64_t walk_key;	 /* the walk's failure: position * 4 + class (0 malformed, 1 output, 2 checksum); ~0 none */
+	uint64_t walk_out;	 /* output bytes of the recorded chunks */
+	uint64_t verify_key;	 /* smallest failure key of the verify step */
+};
+struct csb_framed_table {	/* per data chunk i / per compressed chunk j, in stream order */
+	uint64_t *pos, *out_off;
+	uint32_t *out_len, *crc, *cidx; /* cidx: index j of a compressed chunk, ~0 for a stored one */
+	uint64_t *c_pos, *c_out_off;	/* decoder input: src + 8 + c_pos[j], c_len[j] bytes (varint included) */
+	uint32_t *c_len, *c_produced;
+	int32_t *c_status;
+	struct csb_framed_result *res;
+};
+/* masked CRC-32C per 65536-byte chunk of in[0, n); with flen (sizes of the 32 KiB fragments) also the record sizes */
+int csb_launch_framed_crc(const uint8_t *in, uint64_t n, uint32_t *crc, const uint32_t *flen, uint32_t n_frag, uint32_t *rec,
+			  csb_stream_t s);
+int csb_launch_framed_write(const uint8_t *in, uint64_t n, const uint8_t *slots, uint64_t slot_stride, const uint32_t *flen,
+			    uint32_t n_frag, const uint32_t *crc, const uint32_t *rec, const uint64_t *off, uint8_t *out,
+			    uint64_t *out_length, csb_stream_t s);
+int csb_launch_framed_walk(const uint8_t *src, uint64_t len, uint64_t cap, const struct csb_framed_table *t, csb_stream_t s);
+int csb_launch_framed_verify(const uint8_t *src, uint8_t *dst, uint32_t n_data, const struct csb_framed_table *t,
+			     uint64_t *out_length, int32_t *status, uint64_t *failed_offset, csb_stream_t s);
 
 #ifdef __cplusplus
 }

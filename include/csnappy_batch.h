@@ -21,7 +21,8 @@
  * reference, cl_tester.c:120-165) and >= capacity for decompression.
  * Fast paths engage when base, stride and offsets are multiples of 16.
  *
- * Every function returns 0, CSNAPPY_E_DEVICE or CSNAPPY_E_BAD_ARG; per-block
+ * Every function returns 0, CSNAPPY_E_DEVICE or CSNAPPY_E_BAD_ARG (the framed and container readers also a
+ * stream's decode result); per-block
  * decoder results go to d_status[] / h_status[].
  */
 #ifndef CSNAPPY_B200_CSNAPPY_BATCH_H_
@@ -195,6 +196,76 @@ int csnappy_bc_decompress_host_multi(const void *h_container, uint64_t container
 				     uint32_t page_size, void *h_out, uint64_t out_capacity,
 				     uint64_t *out_length, uint32_t *failed_page,
 				     const int *devices, int n_devices);
+
+/*
+ * Snappy FRAMING FORMAT (the format of .sz files and x-snappy-framed streams): one buffer as a stream of chunks
+ *     [u8 type][u24 LE length][length bytes]
+ * Every data chunk holds at most 65536 uncompressed bytes and a masked CRC-32C of them, so both directions run
+ * chunk-parallel on the device and corruption is detected.
+ *
+ * CRC-32C: Castagnoli polynomial, reflected (0x82F63B78), init ~0, final xor ~0.
+ * mask(crc) = ((crc >> 15) | (crc << 17)) + 0xa282ead8  (mod 2^32).
+ *
+ * Writer (csnappy_framed_compress*): the output is fully determined by (input, wm):
+ *   ff 06 00 00 73 4e 61 50 70 59   stream identifier, once, also for empty input; then for chunk k of the input
+ *   (65536 bytes each, the last one shorter), n_k bytes, c = csnappy_compress(chunk_k, wm) (varint included):
+ *     type 0x00, body [mask(crc32c(chunk_k)) LE][c]        if len(c) < n_k - n_k / 8
+ *     type 0x01, body [mask(crc32c(chunk_k)) LE][chunk_k]  otherwise.
+ *   csnappy_framed_max_length(n) = 10 + 8 * ceil(n / 65536) + n is an exact bound.
+ *
+ * Reader (csnappy_framed_decompress*): walks the chunks from byte 0.
+ *   Zero-length input is an empty stream: 0, no bytes.
+ *   Fewer than 4 header bytes left, or a body running past the end: CSNAPPY_E_DATA_MALFORMED at that chunk.
+ *   The first chunk must be a stream identifier; every 0xff chunk, wherever it appears, must be exactly length 6
+ *   with body "sNaPpY" (concatenated streams are valid).
+ *   0x00 compressed: body >= 5 bytes; the varint32 must be valid and <= 65536; the rest must decode
+ *        (csnappy_decompress_noheader semantics, capacity = the varint) to exactly the varint's length.
+ *   0x01 uncompressed: body >= 4 bytes and at most 65536 data bytes.
+ *   0x02..0x7f (reserved, unskippable): CSNAPPY_E_DATA_MALFORMED.
+ *   0x80..0xfd (reserved, skippable) and 0xfe (padding), any length: skipped.
+ *   Anything else wrong with a data chunk: CSNAPPY_E_DATA_MALFORMED.
+ *   A data chunk whose output would end past out_capacity: CSNAPPY_E_OUTPUT_INSUF.
+ *   A data chunk whose uncompressed bytes do not match its stored masked CRC: CSNAPPY_E_CHECKSUM.
+ * Of the failing chunks, the one with the smallest header position wins.  Framing, varint and capacity failures end
+ * the walk (later chunk boundaries are unknown).  *out_length = the uncompressed bytes of the data chunks before the
+ * winning chunk; they are in dst[0, *out_length) and correct.  Bytes in [*out_length, out_capacity) are unspecified;
+ * nothing is written at or past out_capacity.  *failed_offset = the winning chunk's header position, written only on
+ * a chunk failure (-2, -5, -102); the pointer may be NULL.
+ * Returns 0, CSNAPPY_E_OUTPUT_INSUF, CSNAPPY_E_DATA_MALFORMED, CSNAPPY_E_CHECKSUM, CSNAPPY_E_DEVICE or
+ * CSNAPPY_E_BAD_ARG; a refused argument (wm outside 9..16, a capacity below the bound, a short workspace, a NULL
+ * buffer) returns CSNAPPY_E_BAD_ARG before any device work.
+ */
+#define CSNAPPY_E_CHECKSUM (-102)
+uint64_t csnappy_framed_max_length(uint64_t input_length);
+
+/* Device resident, asynchronous on `stream`.  *d_out_length <- stream length.  out_capacity >=
+ * csnappy_framed_max_length(input_length); d_workspace: csnappy_framed_compress_workspace() bytes, untouched until
+ * the work on `stream` has finished.  Returns 0, CSNAPPY_E_DEVICE or CSNAPPY_E_BAD_ARG. */
+uint64_t csnappy_framed_compress_workspace(uint64_t input_length);
+int csnappy_framed_compress(const void *d_in, uint64_t input_length, void *d_out, uint64_t out_capacity,
+			    uint64_t *d_out_length, int workmem_bytes_power_of_two,
+			    void *d_workspace, uint64_t workspace_bytes, void *stream);
+
+/* Device resident.  *d_status <- the reader's result (0, -2, -5, -102), *d_out_length and *d_failed_offset as above.
+ * The chunk walk runs first and its chunk counts are read back (the call synchronises with `stream` once); the call
+ * returns with decoding and verification enqueued on `stream`.  d_workspace: csnappy_framed_decompress_workspace()
+ * bytes (about 7.5 per byte of src: the chunk tables for the most chunks src_length can hold).  The return value is
+ * 0, CSNAPPY_E_DEVICE or CSNAPPY_E_BAD_ARG. */
+uint64_t csnappy_framed_decompress_workspace(uint64_t src_length);
+int csnappy_framed_decompress(const void *d_src, uint64_t src_length, void *d_dst, uint64_t out_capacity,
+			      uint64_t *d_out_length, int32_t *d_status, uint64_t *d_failed_offset,
+			      void *d_workspace, uint64_t workspace_bytes, void *stream);
+
+/* Host buffers, synchronous.  The whole input and output are staged through the device in one piece (no H2D /
+ * kernel / D2H overlap), and only the valid prefix dst[0, *out_length) is copied back. */
+int csnappy_framed_compress_host(const void *h_in, uint64_t input_length, void *h_out, uint64_t out_capacity,
+				 uint64_t *out_length, int workmem_bytes_power_of_two);
+int csnappy_framed_decompress_host(const void *h_src, uint64_t src_length, void *h_dst, uint64_t out_capacity,
+				   uint64_t *out_length, uint64_t *failed_offset);
+
+/* Masked CRC-32C of each 65536-byte chunk of d_in[0, length) (the last one shorter) -> d_crc[ceil(length / 65536)];
+ * the framing format's checksum, on the device, asynchronous on `stream`. */
+int csnappy_framed_crc32c(const void *d_in, uint64_t length, uint32_t *d_crc, void *stream);
 
 /*
  * Library / device introspection and kernel tuning knobs (used by bench.py and

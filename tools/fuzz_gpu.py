@@ -5,7 +5,9 @@ also gets blocks built to drive the parse through the kernel's rare paths (tests
 sharing in stride-1 and strided windows, in-window copies, the scan end, length and offset boundaries); the decode
 leg gets random streams of every tag form (tests/streams.py), which the compressor never writes.  The container leg
 writes a page container of random page size and length, corrupts its index and payload at random and compares the
-reader with the restated reader (tests/containers.py).
+reader with the restated reader (tests/containers.py).  The framed leg round-trips a random buffer through the framing
+format, compares the stream with the restated writer, corrupts it at random and compares the reader with the restated
+reader (tests/framed.py).
 
     python tools/fuzz_gpu.py [seconds] [seed]
 """
@@ -21,6 +23,7 @@ import csnappy_b200 as cs
 import oracle
 import compress_cases
 import containers
+import framed
 from cases import fuzz_pages
 from streams import random_stream
 
@@ -29,7 +32,7 @@ seed = int(sys.argv[2]) if len(sys.argv) > 2 else 20261017
 chk = oracle.best()
 rng = np.random.default_rng(seed)
 t0 = time.time()
-rounds = blocks = streams = pages_read = 0
+rounds = blocks = streams = pages_read = framed_streams = 0
 while time.time() - t0 < budget:
     size = int(rng.choice([17, 64, 300, 1000, 4096, 4096, 4096, 5000, 16384, 32768]))
     wm = int(rng.integers(9, 17))
@@ -127,10 +130,27 @@ while time.time() - t0 < budget:
     for i, b in want.pages.items():
         assert out[i * page: i * page + len(b)].tobytes() == b, ("container page", page, i)
     pages_read += nr
+    # framed: a random buffer round-trips and its stream equals the restated writer; random corruptions of it give the
+    # restated reader's (rc, out_length, failed_offset) and valid prefix
+    data = containers.mixed_bytes(int(rng.integers(1 << 30)), int(rng.integers(0, 5 * framed.CHUNK)), scale=int(rng.integers(64, 70000)))
+    s = cs.api.framed_compress(data, wm)
+    assert s == framed.write_framed(data, wm), ("framed write", len(data), wm)
+    assert cs.api.framed_decompress(s, len(data)) == (0, data, None), ("framed round trip", len(data))
+    broken = bytearray(s)
+    for _ in range(int(rng.integers(1, 4))):
+        broken[int(rng.integers(0, len(broken)))] ^= 1 << int(rng.integers(0, 8))
+    if rng.random() < 0.2:
+        broken = broken[: int(rng.integers(0, len(broken) + 1))]
+    cap = len(data) - int(rng.integers(0, 2)) * int(rng.integers(0, len(data) + 1))
+    want = framed.read_framed(bytes(broken), cap)
+    rc, out, bad = cs.api.framed_decompress(bytes(broken), cap)
+    assert (rc, len(out), bad) == want.key() and out == want.data, ("framed read", len(data), want.key(), (rc, len(out), bad))
+    framed_streams += 1
     rounds += 1
 cs.set_tuning("compress_lanes", 0)
 cs.set_tuning("decompress_lanes", 0)
 cs.set_tuning("compress_stage_input", 0)
 cs.set_tuning("decompress_stage_input", 0)
 print(f"fuzz ok: {rounds} rounds, {blocks} blocks compressed byte-identically, {streams} streams decoded with identical results, "
-      f"{pages_read} container pages written and read as restated in {time.time() - t0:.0f} s")
+      f"{pages_read} container pages written and read as restated, "
+      f"{framed_streams} framed streams written, corrupted and read as restated in {time.time() - t0:.0f} s")
