@@ -49,6 +49,11 @@ def _declare(L):
         "csnappy_framed_compress_host": (i, [vp, u64, vp, u64, C.POINTER(C.c_uint64), i]),
         "csnappy_framed_decompress_host": (i, [vp, u64, vp, u64, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
         "csnappy_framed_crc32c": (i, [vp, u64, vp, vp]),
+        "csnappy_framed_batch_compress_workspace": (u64, [vp, u32]),
+        "csnappy_framed_batch_compress": (i, [vp, vp, vp, u32, vp, vp, u64, vp, i, vp, u64, vp]),
+        "csnappy_framed_batch_decompress_workspace": (u64, [vp, u32]),
+        "csnappy_framed_batch_decompress": (i, [vp, vp, vp, u32, vp, vp, vp, vp, vp, vp, vp, u64, vp]),
+        "csnappy_framed_batch_decompressed_length": (i, [vp, vp, vp, u32, vp, vp, vp]),
         "csnappy_b200_device_count": (i, []),
         "csnappy_b200_device_ok": (i, []),
         "csnappy_b200_last_error": (C.c_char_p, []),

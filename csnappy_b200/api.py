@@ -14,7 +14,9 @@ Host-buffer batches (numpy / pinned torch tensors, synchronous, pipelined H2D/D2
     batch_compress_fragments_host, batch_decompress_host
 Snappy framing format (64 KiB chunks with masked CRC-32C):
     framed_compress, framed_decompress (host bytes); framed_compress_device, framed_decompress_device,
-    framed_crc32c_device (CUDA tensors, current stream)
+    framed_crc32c_device (CUDA tensors, current stream); many streams in one call: framed_batch_compress,
+    framed_batch_decompress (lists of bytes) and framed_batch_compress_device, framed_batch_decompress_device,
+    framed_batch_decompressed_length_device (CUDA tensors, host offset / length arrays)
 """
 from __future__ import annotations
 
@@ -404,3 +406,121 @@ def framed_crc32c_device(d_in, length: int | None = None, *, crc=None):
     rc = lib().csnappy_framed_crc32c(_ptr(d_in), n, _ptr(crc), _stream_ptr())
     _check(rc, "csnappy_framed_crc32c")
     return crc
+
+
+def _u64(xs) -> np.ndarray:
+    return np.ascontiguousarray(np.asarray(xs, dtype=np.uint64).reshape(-1))
+
+
+def _host_off(a: np.ndarray):
+    return a.ctypes.data if a.size else None
+
+
+def framed_batch_compress_device(d_in, offs, lens, wm: int = CSNAPPY_WORKMEM_BYTES_POWER_OF_TWO, *, out_off=None,
+                                 out=None):
+    """Many framed streams written in one call: stream i is d_in[offs[i], offs[i] + lens[i]) (HOST sequences).
+    Slot i of `out` starts at out_off[i] (None: the running sum of framed_max_length(lens[j]), j < i).
+    Returns (out uint8 CUDA tensor, out_off numpy uint64, out_len int64 CUDA tensor), asynchronous on the current
+    stream."""
+    import torch
+
+    h_off, h_len = _u64(offs), _u64(lens)
+    n = len(h_len)
+    m = np.array([framed_max_length(int(x)) for x in h_len], dtype=np.uint64)
+    h_out = _u64(np.concatenate((np.zeros(1, np.uint64), np.cumsum(m)[:-1]))) if out_off is None else _u64(out_off)
+    cap = int((h_out + m).max()) if n else 0
+    if out is None:
+        out = torch.empty(max(cap, 1), dtype=torch.uint8, device=d_in.device)
+    out_len = torch.empty(max(n, 1), dtype=torch.int64, device=d_in.device)
+    ws_bytes = lib().csnappy_framed_batch_compress_workspace(_host_off(h_len), n)
+    ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=d_in.device)
+    rc = lib().csnappy_framed_batch_compress(_ptr(d_in), _host_off(h_off), _host_off(h_len), n, _ptr(out),
+                                             None if out_off is None else _host_off(h_out), out.numel(), _ptr(out_len),
+                                             wm, _ptr(ws), ws_bytes, _stream_ptr())
+    _check(rc, "csnappy_framed_batch_compress")
+    return out, h_out, out_len  # the workspace is freed in stream order, as in framed_compress_device
+
+
+def framed_batch_decompressed_length_device(d_src, offs, lens):
+    """Declared decompressed length of every framed stream (the chunk walk, no decoding): returns (length int64,
+    status int32) CUDA tensors; status -5 where the walk finds a framing failure (length then counts the chunks before
+    it)."""
+    import torch
+
+    h_off, h_len = _u64(offs), _u64(lens)
+    n = len(h_len)
+    length = torch.empty(max(n, 1), dtype=torch.int64, device=d_src.device)
+    status = torch.empty(max(n, 1), dtype=torch.int32, device=d_src.device)
+    rc = lib().csnappy_framed_batch_decompressed_length(_ptr(d_src), _host_off(h_off), _host_off(h_len), n, _ptr(length),
+                                                        _ptr(status), _stream_ptr())
+    _check(rc, "csnappy_framed_batch_decompressed_length")
+    return length, status
+
+
+def framed_batch_decompress_device(d_src, offs, lens, caps, *, dst_off=None, dst=None, failed_offset=None):
+    """Many framed streams read in one call (the call waits once for the chunk walk of the whole batch).  Output i
+    goes to dst[dst_off[i], + caps[i]) (dst_off None: the running sum of caps).  Returns (dst uint8 CUDA tensor,
+    dst_off numpy uint64, result int64 CUDA tensor [3, n] = out_len, rc, failed_offset); failed_offset (default
+    prefilled with -1) is written only for streams that fail."""
+    import torch
+
+    h_off, h_len, h_cap = _u64(offs), _u64(lens), _u64(caps)
+    n = len(h_len)
+    h_dst = _u64(np.concatenate((np.zeros(1, np.uint64), np.cumsum(h_cap)[:-1]))) if dst_off is None else _u64(dst_off)
+    if dst is None:
+        dst = torch.empty(max(int((h_dst + h_cap).max()) if n else 0, 1), dtype=torch.uint8, device=d_src.device)
+    result = torch.empty((3, max(n, 1)), dtype=torch.int64, device=d_src.device)
+    if failed_offset is None:
+        result[2].fill_(-1)
+    else:
+        result[2].copy_(failed_offset)
+    status = torch.zeros(max(n, 1), dtype=torch.int32, device=d_src.device)
+    ws_bytes = lib().csnappy_framed_batch_decompress_workspace(_host_off(h_len), n)
+    ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=d_src.device)
+    rc = lib().csnappy_framed_batch_decompress(_ptr(d_src), _host_off(h_off), _host_off(h_len), n, _ptr(dst),
+                                               _host_off(h_dst), _host_off(h_cap), result[0].data_ptr(), _ptr(status),
+                                               result[2].data_ptr(), _ptr(ws), ws_bytes, _stream_ptr())
+    _check(rc, "csnappy_framed_batch_decompress")
+    result[1].copy_(status)
+    return dst, h_dst, result
+
+
+def _stage(bufs):
+    """Byte strings -> (one uint8 CUDA tensor, offsets, lengths)."""
+    import torch
+
+    lens = [len(b) for b in bufs]
+    offs = np.concatenate(([0], np.cumsum(lens)[:-1])).astype(np.uint64) if bufs else np.zeros(0, np.uint64)
+    host = np.frombuffer(b"".join(bytes(b) for b in bufs) or b"\0", dtype=np.uint8)
+    return torch.from_numpy(host.copy()).cuda(), offs, lens
+
+
+def framed_batch_compress(bufs, wm: int = CSNAPPY_WORKMEM_BYTES_POWER_OF_TWO) -> list[bytes]:
+    """A list of byte strings -> their framed streams, written in one device call."""
+    import torch
+
+    if not bufs:
+        return []
+    d, offs, lens = _stage(bufs)
+    out, out_off, out_len = framed_batch_compress_device(d, offs, lens, wm)
+    torch.cuda.current_stream().synchronize()
+    raw, ol = out.cpu().numpy(), out_len.cpu().tolist()
+    return [raw[int(o):int(o) + n].tobytes() for o, n in zip(out_off, ol)]
+
+
+def framed_batch_decompress(bufs, caps=None):
+    """A list of framed streams -> [(rc, valid prefix, failed_offset or None)], read in one device call.  caps=None:
+    each stream's capacity is its declared length (framed_batch_decompressed_length_device)."""
+    import torch
+
+    if not bufs:
+        return []
+    d, offs, lens = _stage(bufs)
+    if caps is None:
+        length, _ = framed_batch_decompressed_length_device(d, offs, lens)
+        caps = length[: len(bufs)].cpu().tolist()
+    dst, dst_off, res = framed_batch_decompress_device(d, offs, lens, caps)
+    torch.cuda.current_stream().synchronize()
+    raw, r = dst.cpu().numpy(), res.cpu().tolist()
+    return [(int(r[1][i]), raw[int(dst_off[i]):int(dst_off[i]) + r[0][i]].tobytes(), r[2][i] if r[1][i] else None)
+            for i in range(len(bufs))]

@@ -2083,3 +2083,359 @@ out:
 	ctx_release(c);
 	return rc;
 }
+
+/* ---- many framed streams in one call (csnappy_framed_batch_*) --------------------------------------------------------
+ * Exactly N independent single calls, with a launch count that does not grow with N.
+ * Writer: the host lays out every stream's chunks and their 32 KiB fragments (a chunk's short last fragment takes the
+ * short-chunk table rule, as csnappy_compress(chunk) does); one compress launch over all fragments, one warp per chunk
+ * for CRC and record size, one scan over all records, one warp per chunk to write, one thread per stream for the
+ * identifier and the length.
+ * Reader: one thread per stream walks its headers into its own table region; scans of the per-stream counts and a
+ * compaction make the tables contiguous; the host reads the two totals back (the one synchronisation); then one decode
+ * launch, one warp per data chunk to verify and one thread per stream for the result.                               */
+#define FRAMED_BATCH_NONE (~(uint64_t)0)
+
+/* writer workspace after the fragment slots: device-written tables, then the host-built ones (one upload) */
+enum { WB_FLEN, WB_CRC, WB_REC, WB_OFF, WB_CTR, WB_FIN, WB_FOFF, WB_CIN, WB_CLEN, WB_CSTREAM, WB_CFRAG, WB_SOUT, WB_SFIRST, WB_END };
+
+static uint64_t framed_batch_compress_layout(uint64_t F, uint64_t K, uint64_t n, uint64_t o[WB_END + 1])
+{
+	const uint64_t per[WB_END] = {F * 4, K * 4, K * 4, (K + 1) * 8, 256, F * 4, F * 8, K * 8, K * 4, K * 4, K * 4, n * 8, (n + 1) * 4};
+	uint64_t p = al256(F * SLOT_STRIDE_32K);
+	int i;
+	for (i = 0; i < WB_END; i++) {
+		o[i] = p;
+		p = al256(p + per[i]);
+	}
+	o[WB_END] = p;
+	return p;
+}
+
+/* fragments and chunks of a batch; 0 when a stream is too long or the fragments leave uint32 (chunks <= fragments) */
+static int framed_batch_counts(const uint64_t *h_len, uint32_t n, uint64_t *F, uint64_t *K)
+{
+	uint32_t i;
+	*F = *K = 0;
+	for (i = 0; i < n; i++) {
+		if (h_len[i] > FRAMED_MAX_INPUT)
+			return 0;
+		*F += (h_len[i] + CSB_FRAGMENT_MAX - 1) / CSB_FRAGMENT_MAX;
+		*K += chunks_of(h_len[i]);
+		if (*F > 0xffffffffull)
+			return 0;
+	}
+	return 1;
+}
+
+uint64_t csnappy_framed_batch_compress_workspace(const uint64_t *h_in_len, uint32_t n_streams)
+{
+	uint64_t F, K, o[WB_END + 1];
+	if ((n_streams && !h_in_len) || !framed_batch_counts(h_in_len, n_streams, &F, &K))
+		return FRAMED_BATCH_NONE;
+	return framed_batch_compress_layout(F, K, n_streams, o);
+}
+
+int csnappy_framed_batch_compress(const void *d_in, const uint64_t *h_in_off, const uint64_t *h_in_len, uint32_t n_streams,
+				  void *d_out, const uint64_t *h_out_off, uint64_t out_capacity, uint64_t *d_out_len,
+				  int workmem_bytes_power_of_two, void *d_workspace, uint64_t workspace_bytes, void *stream)
+{
+	uint64_t F, K, o[WB_END + 1], at = 0, f = 0, k = 0, total_in = 0;
+	uint8_t *ws = (uint8_t *)d_workspace, *tab;
+	csb_stream_t s = (csb_stream_t)stream;
+	struct csb_framed_batch_wtable t;
+	struct csb_compress_args a;
+	uint32_t i;
+	int e;
+	if (workmem_bytes_power_of_two < 9 || workmem_bytes_power_of_two > 16)
+		return set_err("workmem_bytes_power_of_two outside 9..16", 0);
+	if (n_streams == 0)
+		return 0;
+	if (!h_in_off || !h_in_len || !d_out || !d_out_len || !d_workspace)
+		return set_err("null buffer", 0);
+	if (!framed_batch_counts(h_in_len, n_streams, &F, &K))
+		return set_err("a stream longer than (2^32 - 2) * 32768 bytes, or more than 2^32 - 1 fragments", 0);
+	for (i = 0; i < n_streams; i++) {
+		const uint64_t base = h_out_off ? h_out_off[i] : at, m = csnappy_framed_max_length(h_in_len[i]);
+		if (base > out_capacity || m > out_capacity - base)
+			return set_err("output slot ending past out_capacity", 0);
+		at = base + m;
+		total_in += h_in_len[i];
+	}
+	if (total_in && !d_in)
+		return set_err("null buffer", 0);
+	if (workspace_bytes < framed_batch_compress_layout(F, K, n_streams, o))
+		return set_err("workspace smaller than csnappy_framed_batch_compress_workspace()", 0);
+	/* host image of the tables [o[WB_FIN], o[WB_END]) */
+	tab = (uint8_t *)malloc((size_t)(o[WB_END] - o[WB_FIN]));
+	if (!tab)
+		return set_err("host table", (int)cudaErrorMemoryAllocation);
+	{
+#define HT(idx, type) ((type *)(tab + (o[idx] - o[WB_FIN])))
+		uint32_t *fin = HT(WB_FIN, uint32_t), *c_len = HT(WB_CLEN, uint32_t), *c_stream = HT(WB_CSTREAM, uint32_t);
+		uint32_t *c_frag = HT(WB_CFRAG, uint32_t), *s_first = HT(WB_SFIRST, uint32_t);
+		uint64_t *foff = HT(WB_FOFF, uint64_t), *c_in = HT(WB_CIN, uint64_t), *s_out = HT(WB_SOUT, uint64_t);
+#undef HT
+		at = 0;
+		for (i = 0; i < n_streams; i++) {
+			const uint64_t base = h_in_off[i], n = h_in_len[i];
+			uint64_t c;
+			s_out[i] = h_out_off ? h_out_off[i] : at;
+			s_first[i] = (uint32_t)k;
+			at += csnappy_framed_max_length(n);
+			for (c = 0; c < n; c += FRAMED_CHUNK) {
+				const uint32_t m = n - c < FRAMED_CHUNK ? (uint32_t)(n - c) : (uint32_t)FRAMED_CHUNK;
+				uint32_t q;
+				c_in[k] = base + c;
+				c_len[k] = m;
+				c_stream[k] = i;
+				c_frag[k] = (uint32_t)f;
+				for (q = 0; q < m; q += CSB_FRAGMENT_MAX) {
+					foff[f] = base + c + q;
+					fin[f] = m - q < CSB_FRAGMENT_MAX ? m - q : CSB_FRAGMENT_MAX;
+					f++;
+				}
+				k++;
+			}
+		}
+		s_first[n_streams] = (uint32_t)k;
+	}
+	/* pageable source: the copy is staged before the call returns, the table can be freed right after */
+	e = (int)cudaMemcpyAsync(ws + o[WB_FIN], tab, (size_t)(o[WB_END] - o[WB_FIN]), cudaMemcpyHostToDevice, (cudaStream_t)s);
+	free(tab);
+	if (e)
+		return set_err("H2D chunk tables", e);
+	t.flen = (const uint32_t *)(ws + o[WB_FLEN]);
+	t.c_in = (const uint64_t *)(ws + o[WB_CIN]);
+	t.c_len = (const uint32_t *)(ws + o[WB_CLEN]);
+	t.c_stream = (const uint32_t *)(ws + o[WB_CSTREAM]);
+	t.c_frag = (const uint32_t *)(ws + o[WB_CFRAG]);
+	t.crc = (uint32_t *)(ws + o[WB_CRC]);
+	t.rec = (uint32_t *)(ws + o[WB_REC]);
+	t.off = (const uint64_t *)(ws + o[WB_OFF]);
+	t.s_out = (const uint64_t *)(ws + o[WB_SOUT]);
+	t.s_first = (const uint32_t *)(ws + o[WB_SFIRST]);
+	if (F) {
+		fill_compress_args(&a);
+		a.in = (const uint8_t *)d_in;
+		a.in_off = (const uint64_t *)(ws + o[WB_FOFF]);
+		a.in_len = (const uint32_t *)(ws + o[WB_FIN]);
+		a.n_blocks = (uint32_t)F;
+		a.out = ws;
+		a.out_stride = SLOT_STRIDE_32K;
+		a.out_len = (uint32_t *)(ws + o[WB_FLEN]);
+		a.wm = workmem_bytes_power_of_two;
+		a.flags = CSNAPPY_BATCH_SHRINK_TABLE; /* applies to fragments below 32768 bytes: a chunk's short last one */
+		a.counter = (uint32_t *)(ws + o[WB_CTR]);
+		if ((e = csb_launch_compress(&a, s)))
+			return set_err("compress launch", e);
+		if ((e = csb_launch_framed_batch_crc((const uint8_t *)d_in, (uint32_t)K, &t, s)))
+			return set_err("crc launch", e);
+	}
+	if ((e = csb_launch_scan(t.rec, (uint32_t)K, (uint64_t *)(ws + o[WB_OFF]), s)))
+		return set_err("scan launch", e);
+	e = csb_launch_framed_batch_write((const uint8_t *)d_in, (uint32_t)K, n_streams, ws, SLOT_STRIDE_32K, &t,
+					  (uint8_t *)d_out, d_out_len, s);
+	return e ? set_err("framed write launch", e) : 0;
+}
+
+/* reader workspace: per-stream table (uploaded) and results, the two scans and the totals, then the region tables and
+ * the compacted tables for D = sum(src_len / 8 + 1) data chunks (a data chunk takes at least 8 bytes of its stream),
+ * then the decoder's block counter */
+enum { RB_SSRC, RB_SLEN, RB_SDST, RB_SCAP, RB_SREG, RB_ND, RB_NC, RB_WKEY, RB_WOUT, RB_VKEY, RB_DBASE, RB_CBASE, RB_TOT,
+       RB_RPOS, RB_ROUT, RB_RLEN, RB_RCRC, RB_RCIDX, RB_RPLEN, RB_POS, RB_OUTOFF, RB_OUTLEN, RB_CRC, RB_CIDX, RB_STREAM,
+       RB_CPOS, RB_COUTOFF, RB_CLEN, RB_CPROD, RB_CSTATUS, RB_CTR, RB_END };
+
+static uint64_t framed_batch_decompress_layout(uint64_t D, uint64_t n, uint8_t *ws, uint64_t o[RB_END + 1],
+					       struct csb_framed_batch_rtable *t)
+{
+	const uint64_t per[RB_END] = {n * 8, n * 8, n * 8, n * 8, n * 8, n * 4, n * 4, n * 8, n * 8, n * 8, (n + 1) * 8,
+				      (n + 1) * 8, 16, D * 8, D * 8, D * 4, D * 4, D * 4, D * 4, D * 8, D * 8, D * 4,
+				      D * 4, D * 4, D * 4, D * 8, D * 8, D * 4, D * 4, D * 4, 256};
+	uint64_t p = 0;
+	int i;
+	for (i = 0; i < RB_END; i++) {
+		o[i] = p;
+		p = al256(p + per[i]);
+	}
+	o[RB_END] = p;
+	if (t) {
+#define RT(idx, type) ((type *)(ws + o[idx]))
+		t->s_src = RT(RB_SSRC, const uint64_t);
+		t->s_len = RT(RB_SLEN, const uint64_t);
+		t->s_dst = RT(RB_SDST, const uint64_t);
+		t->s_cap = RT(RB_SCAP, const uint64_t);
+		t->s_reg = RT(RB_SREG, const uint64_t);
+		t->nd = RT(RB_ND, uint32_t);
+		t->nc = RT(RB_NC, uint32_t);
+		t->walk_key = RT(RB_WKEY, uint64_t);
+		t->walk_out = RT(RB_WOUT, uint64_t);
+		t->verify_key = RT(RB_VKEY, uint64_t);
+		t->d_base = RT(RB_DBASE, uint64_t);
+		t->c_base = RT(RB_CBASE, uint64_t);
+		t->totals = RT(RB_TOT, uint64_t);
+		t->r_pos = RT(RB_RPOS, uint64_t);
+		t->r_out = RT(RB_ROUT, uint64_t);
+		t->r_len = RT(RB_RLEN, uint32_t);
+		t->r_crc = RT(RB_RCRC, uint32_t);
+		t->r_cidx = RT(RB_RCIDX, uint32_t);
+		t->r_plen = RT(RB_RPLEN, uint32_t);
+		t->pos = RT(RB_POS, uint64_t);
+		t->out_off = RT(RB_OUTOFF, uint64_t);
+		t->out_len = RT(RB_OUTLEN, uint32_t);
+		t->crc = RT(RB_CRC, uint32_t);
+		t->cidx = RT(RB_CIDX, uint32_t);
+		t->stream = RT(RB_STREAM, uint32_t);
+		t->c_pos = RT(RB_CPOS, uint64_t);
+		t->c_out_off = RT(RB_COUTOFF, uint64_t);
+		t->c_len = RT(RB_CLEN, uint32_t);
+		t->c_produced = RT(RB_CPROD, uint32_t);
+		t->c_status = RT(RB_CSTATUS, int32_t);
+#undef RT
+	}
+	return p;
+}
+
+/* table entries of a batch (sum of src_len / 8 + 1); 0 when a stream is longer than 2^35 bytes or D leaves uint32 */
+static int framed_batch_entries(const uint64_t *h_len, uint32_t n, uint64_t *D)
+{
+	uint32_t i;
+	*D = 0;
+	for (i = 0; i < n; i++) {
+		if (h_len[i] > FRAMED_MAX_SRC)
+			return 0;
+		*D += h_len[i] / 8 + 1;
+		if (*D > 0xffffffffull)
+			return 0;
+	}
+	return 1;
+}
+
+uint64_t csnappy_framed_batch_decompress_workspace(const uint64_t *h_src_len, uint32_t n_streams)
+{
+	uint64_t D, o[RB_END + 1];
+	if ((n_streams && !h_src_len) || !framed_batch_entries(h_src_len, n_streams, &D))
+		return FRAMED_BATCH_NONE;
+	return framed_batch_decompress_layout(D, n_streams, NULL, o, NULL);
+}
+
+int csnappy_framed_batch_decompress(const void *d_src, const uint64_t *h_src_off, const uint64_t *h_src_len,
+				    uint32_t n_streams, void *d_dst, const uint64_t *h_dst_off, const uint64_t *h_dst_cap,
+				    uint64_t *d_out_len, int32_t *d_status, uint64_t *d_failed_offset, void *d_workspace,
+				    uint64_t workspace_bytes, void *stream)
+{
+	struct csb_framed_batch_rtable t;
+	struct csb_decompress_args a;
+	uint64_t D, o[RB_END + 1], totals[2], reg = 0, total_src = 0, total_cap = 0, *h;
+	uint8_t *ws = (uint8_t *)d_workspace;
+	cudaStream_t s = (cudaStream_t)stream;
+	const uint8_t *src = (const uint8_t *)d_src;
+	uint32_t i;
+	int e;
+	if (n_streams == 0)
+		return 0;
+	if (!h_src_off || !h_src_len || !h_dst_off || !h_dst_cap || !d_out_len || !d_status || !d_workspace)
+		return set_err("null buffer", 0);
+	if (!framed_batch_entries(h_src_len, n_streams, &D))
+		return set_err("a stream longer than 2^35 bytes, or more than 2^32 - 1 chunk table entries", 0);
+	for (i = 0; i < n_streams; i++) {
+		total_src |= h_src_len[i];
+		total_cap |= h_dst_cap[i];
+	}
+	if ((total_src && !d_src) || (total_cap && !d_dst))
+		return set_err("null buffer", 0);
+	if (workspace_bytes < framed_batch_decompress_layout(D, n_streams, ws, o, &t))
+		return set_err("workspace smaller than csnappy_framed_batch_decompress_workspace()", 0);
+	/* the per-stream table [o[RB_SSRC], o[RB_ND]): source offset, length, output offset, capacity, table region */
+	h = (uint64_t *)malloc((size_t)(o[RB_ND] - o[RB_SSRC]));
+	if (!h)
+		return set_err("host table", (int)cudaErrorMemoryAllocation);
+	for (i = 0; i < n_streams; i++) {
+		h[(o[RB_SSRC] / 8) + i] = h_src_off[i];
+		h[(o[RB_SLEN] / 8) + i] = h_src_len[i];
+		h[(o[RB_SDST] / 8) + i] = h_dst_off[i];
+		h[(o[RB_SCAP] / 8) + i] = h_dst_cap[i];
+		h[(o[RB_SREG] / 8) + i] = reg;
+		reg += h_src_len[i] / 8 + 1;
+	}
+	e = (int)cudaMemcpyAsync(ws + o[RB_SSRC], h, (size_t)(o[RB_ND] - o[RB_SSRC]), cudaMemcpyHostToDevice, s);
+	free(h);
+	if (e)
+		return set_err("H2D stream table", e);
+	if ((e = csb_launch_framed_batch_walk(src, n_streams, &t, NULL, NULL, (csb_stream_t)s)))
+		return set_err("framed walk launch", e);
+	if ((e = csb_launch_scan(t.nd, n_streams, t.d_base, (csb_stream_t)s)) ||
+	    (e = csb_launch_scan(t.nc, n_streams, t.c_base, (csb_stream_t)s)))
+		return set_err("scan launch", e);
+	if ((e = csb_launch_framed_batch_compact(n_streams, &t, (csb_stream_t)s)))
+		return set_err("compact launch", e);
+	/* the only synchronisation: the batch totals size the launches below */
+	if ((e = (int)cudaMemcpyAsync(totals, t.totals, sizeof(totals), cudaMemcpyDeviceToHost, s)) ||
+	    (e = (int)cudaStreamSynchronize(s)))
+		return set_err("D2H chunk totals", e);
+	if (totals[1]) {
+		fill_decompress_args(&a);
+		a.in = src + 8; /* block j = the body behind chunk j's header and CRC */
+		a.in_off = t.c_pos;
+		a.in_len = t.c_len;
+		a.n_blocks = (uint32_t)totals[1];
+		a.out = (uint8_t *)d_dst;
+		a.out_off = t.c_out_off;
+		a.uniform_cap = CSB_FRAMED_CHUNK; /* WITH_HEADER: the capacity becomes the varint's value, <= 65536 */
+		a.out_len = t.c_produced;
+		a.status = t.c_status;
+		a.flags = CSNAPPY_BATCH_WITH_HEADER;
+		a.counter = (uint32_t *)(ws + o[RB_CTR]);
+		if ((e = csb_launch_decompress(&a, (csb_stream_t)s)))
+			return set_err("decompress launch", e);
+	}
+	e = csb_launch_framed_batch_verify(src, (uint8_t *)d_dst, (uint32_t)totals[0], n_streams, &t, d_out_len, d_status,
+					   d_failed_offset, (csb_stream_t)s);
+	return e ? set_err("framed verify launch", e) : 0;
+}
+
+int csnappy_framed_batch_decompressed_length(const void *d_src, const uint64_t *h_src_off, const uint64_t *h_src_len,
+					     uint32_t n_streams, uint64_t *d_length, int32_t *d_status, void *stream)
+{
+	struct csb_framed_batch_rtable t;
+	cudaStream_t s = (cudaStream_t)stream;
+	uint64_t *h, total_src = 0;
+	void *d_tab = NULL;
+	uint32_t i;
+	int e;
+	if (n_streams == 0)
+		return 0;
+	if (!h_src_off || !h_src_len || !d_length || !d_status)
+		return set_err("null buffer", 0);
+	for (i = 0; i < n_streams; i++) {
+		if (h_src_len[i] > FRAMED_MAX_SRC)
+			return set_err("a stream longer than 2^35 bytes", 0);
+		total_src |= h_src_len[i];
+	}
+	if (total_src && !d_src)
+		return set_err("null buffer", 0);
+	/* the offsets and lengths go to a stream-ordered allocation, freed behind the walk */
+	h = (uint64_t *)malloc((size_t)n_streams * 16);
+	if (!h)
+		return set_err("host table", (int)cudaErrorMemoryAllocation);
+	memcpy(h, h_src_off, (size_t)n_streams * 8);
+	memcpy(h + n_streams, h_src_len, (size_t)n_streams * 8);
+	e = (int)cudaMallocAsync(&d_tab, (size_t)n_streams * 16, s);
+	if (!e)
+		e = (int)cudaMemcpyAsync(d_tab, h, (size_t)n_streams * 16, cudaMemcpyHostToDevice, s);
+	free(h);
+	if (e) {
+		if (d_tab)
+			cudaFreeAsync(d_tab, s);
+		return set_err("H2D stream table", e);
+	}
+	memset(&t, 0, sizeof(t));
+	t.s_src = (const uint64_t *)d_tab;
+	t.s_len = (const uint64_t *)d_tab + n_streams;
+	e = csb_launch_framed_batch_walk((const uint8_t *)d_src, n_streams, &t, d_length, d_status, (csb_stream_t)s);
+	if (e) {
+		cudaFreeAsync(d_tab, s);
+		return set_err("framed length walk launch", e);
+	}
+	e = (int)cudaFreeAsync(d_tab, s);
+	return e ? set_err("cudaFreeAsync(stream table)", e) : 0;
+}

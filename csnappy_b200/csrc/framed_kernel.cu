@@ -225,12 +225,15 @@ enum : uint32_t { kClassMalformed = 0, kClassOutput = 1, kClassChecksum = 2 };
 __device__ __forceinline__ uint32_t get_u24(const uint8_t *p) { return p[0] | (uint32_t)p[1] << 8 | (uint32_t)p[2] << 16; }
 __device__ __forceinline__ uint32_t get_u32(const uint8_t *p) { return get_u24(p) | (uint32_t)p[3] << 24; }
 
-// The chain of chunk headers, one thread.  Records every data chunk before the first failure the walk can detect
-// itself (framing, identifier, varint, data length, capacity) and that failure's key position * 4 + class.
-__global__ void framed_walk_kernel(const uint8_t *__restrict__ src, uint64_t len, uint64_t cap, struct csb_framed_table t)
+// The reader's rules for the chain of chunk headers of ONE stream src[0, len) with output capacity cap, shared by the
+// single and the batched walk.  Calls rec(pos, out, olen, crc, plen, compressed) for every data chunk before the first
+// failure the walk can detect itself (framing, identifier, varint, data length, capacity) and returns that failure's
+// key position * 4 + class (kNone if there is none); *out_total = the output bytes of the recorded chunks.
+template <class Rec>
+__device__ __forceinline__ uint64_t walk_chunks(const uint8_t *__restrict__ src, uint64_t len, uint64_t cap,
+						uint64_t *out_total, Rec &&rec)
 {
 	uint64_t pos = 0, out = 0, key = kNone;
-	uint32_t nd = 0, nc = 0;
 	while (pos < len) {
 		if (len - pos < 4) {
 			key = pos * 4 + kClassMalformed;
@@ -284,20 +287,7 @@ __global__ void framed_walk_kernel(const uint8_t *__restrict__ src, uint64_t len
 				key = pos * 4 + kClassOutput;
 				break;
 			}
-			t.pos[nd] = pos;
-			t.out_off[nd] = out;
-			t.out_len[nd] = olen;
-			t.crc[nd] = get_u32(h + 4);
-			if (type == 0u) {
-				t.cidx[nd] = nc;
-				t.c_pos[nc] = pos;
-				t.c_len[nc] = plen;
-				t.c_out_off[nc] = out;
-				++nc;
-			} else {
-				t.cidx[nd] = 0xffffffffu;
-			}
-			++nd;
+			rec(pos, out, olen, get_u32(h + 4), plen, type == 0u);
 			out += olen;
 		} else if (type <= 0x7fu) {  // reserved unskippable
 			key = pos * 4 + kClassMalformed;
@@ -306,6 +296,32 @@ __global__ void framed_walk_kernel(const uint8_t *__restrict__ src, uint64_t len
 		// 0x80..0xfe: skippable / padding
 		pos = body + blen;
 	}
+	*out_total = out;
+	return key;
+}
+
+// The chain of chunk headers, one thread: the chunk table of csb_framed_table and the result words.
+__global__ void framed_walk_kernel(const uint8_t *__restrict__ src, uint64_t len, uint64_t cap, struct csb_framed_table t)
+{
+	uint64_t out;
+	uint32_t nd = 0, nc = 0;
+	const uint64_t key = walk_chunks(src, len, cap, &out,
+					 [&](uint64_t pos, uint64_t o, uint32_t olen, uint32_t crc, uint32_t plen, bool comp) {
+						 t.pos[nd] = pos;
+						 t.out_off[nd] = o;
+						 t.out_len[nd] = olen;
+						 t.crc[nd] = crc;
+						 if (comp) {
+							 t.cidx[nd] = nc;
+							 t.c_pos[nc] = pos;
+							 t.c_len[nc] = plen;
+							 t.c_out_off[nc] = o;
+							 ++nc;
+						 } else {
+							 t.cidx[nd] = 0xffffffffu;
+						 }
+						 ++nd;
+					 });
 	t.res->n_data = nd;
 	t.res->n_comp = nc;
 	t.res->walk_key = key;
@@ -379,6 +395,216 @@ __global__ void framed_finish_kernel(struct csb_framed_table t, uint64_t *__rest
 		*failed_offset = pos;
 }
 
+// ---- many streams in one call (csnappy_framed_batch_*) --------------------------------------------------------------
+// Writer.  One warp per chunk of every stream: masked CRC and record size, as framed_crc_kernel, with the chunk's input
+// and fragments taken from the host-built chunk table.
+__global__ void __launch_bounds__(256) framed_batch_crc_kernel(const uint8_t *__restrict__ in, uint32_t n_chunks,
+							       struct csb_framed_batch_wtable t)
+{
+	__shared__ CrcTables T;
+	load_crc_tables(T);
+	const uint32_t warps = (gridDim.x * blockDim.x) >> 5;
+	for (uint32_t k = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; k < n_chunks; k += warps) {
+		const uint32_t m = t.c_len[k];
+		const uint32_t c = warp_crc32c(T, in + t.c_in[k], m);
+		if ((threadIdx.x & 31u) == 0) {
+			const uint32_t f = t.c_frag[k];
+			const uint32_t f1 = m > CSB_FRAGMENT_MAX ? t.flen[f + 1] : 0u;
+			const uint32_t clen = varint_len(m) + t.flen[f] + f1;
+			t.crc[k] = c;
+			t.rec[k] = 8u + (clen < m - m / 8 ? clen : m);
+		}
+	}
+}
+
+// One warp per chunk: header, CRC and payload of chunk k at its stream's slot + 10 + (off[k] - off[the stream's first
+// chunk]).  Then one thread per stream writes its identifier (empty streams too) and out_length.
+__global__ void __launch_bounds__(256) framed_batch_write_kernel(const uint8_t *__restrict__ in, uint32_t n_chunks,
+								 uint32_t n_streams, const uint8_t *__restrict__ slots,
+								 uint64_t slot_stride, struct csb_framed_batch_wtable t,
+								 uint8_t *__restrict__ out, uint64_t *__restrict__ out_length)
+{
+	const uint32_t lane = threadIdx.x & 31u;
+	const uint32_t warps = (gridDim.x * blockDim.x) >> 5;
+	for (uint32_t k = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; k < n_chunks; k += warps) {
+		const uint32_t m = t.c_len[k], st = t.c_stream[k], rec = t.rec[k];
+		const uint32_t body = rec - 4u;
+		const bool comp = rec != 8u + m;  // a stored record is 8 + m bytes, a compressed one fewer
+		uint8_t *dst = out + t.s_out[st] + 10u + (t.off[k] - t.off[t.s_first[st]]);
+		const uint32_t c = t.crc[k];
+		if (lane < 8) {
+			const uint32_t hdr = lane < 4 ? ((comp ? 0x00u : 0x01u) | (body << 8)) : c;
+			dst[lane] = (uint8_t)(hdr >> (8 * (lane & 3u)));
+		}
+		if (!comp) {
+			warp_copy(dst + 8, in + t.c_in[k], m);
+			continue;
+		}
+		const uint32_t hv = varint_len(m);
+		if (lane < hv)
+			dst[8 + lane] = (uint8_t)(((m >> (7 * lane)) & 0x7fu) | (lane + 1 < hv ? 0x80u : 0u));
+		const uint32_t f = t.c_frag[k], f0 = t.flen[f];
+		warp_copy(dst + 8 + hv, slots + (uint64_t)f * slot_stride, f0);
+		if (m > CSB_FRAGMENT_MAX)
+			warp_copy(dst + 8 + hv + f0, slots + (uint64_t)(f + 1) * slot_stride, t.flen[f + 1]);
+	}
+	const uint32_t threads = gridDim.x * blockDim.x;
+	for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_streams; i += threads) {
+		uint8_t *o = out + t.s_out[i];
+		// ff 06 00 00 73 4e 61 50 70 59: type 0xff, length 6, "sNaPpY"
+		for (uint32_t b = 0; b < 10; ++b)
+			o[b] = (uint8_t)(b < 8 ? 0x50614e73000006ffull >> (8 * b) : 0x5970u >> (8 * (b - 8)));
+		out_length[i] = 10u + (t.off[t.s_first[i + 1]] - t.off[t.s_first[i]]);
+	}
+}
+
+// Reader.  One thread per stream walks its chunk headers (walk_chunks) into its own region of the r_* tables.  With
+// `length` set it is the decompressed_length walk instead: unbounded capacity, no table writes, the declared data
+// length and 0 / -5 per stream.
+__global__ void __launch_bounds__(128) framed_batch_walk_kernel(const uint8_t *__restrict__ src, uint32_t n_streams,
+								struct csb_framed_batch_rtable t, uint64_t *__restrict__ length,
+								int32_t *__restrict__ status)
+{
+	const uint32_t threads = gridDim.x * blockDim.x;
+	for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_streams; i += threads) {
+		const uint8_t *s = src + t.s_src[i];
+		uint64_t out;
+		if (length) {
+			const uint64_t key = walk_chunks(s, t.s_len[i], kNone, &out,
+							 [](uint64_t, uint64_t, uint32_t, uint32_t, uint32_t, bool) {});
+			length[i] = out;
+			status[i] = key == kNone ? 0 : -5;
+			continue;
+		}
+		const uint64_t reg = t.s_reg[i];
+		uint32_t nd = 0, nc = 0;
+		const uint64_t key = walk_chunks(s, t.s_len[i], t.s_cap[i], &out,
+						 [&](uint64_t pos, uint64_t o, uint32_t olen, uint32_t crc, uint32_t plen, bool comp) {
+							 const uint64_t r = reg + nd;
+							 t.r_pos[r] = pos;
+							 t.r_out[r] = o;
+							 t.r_len[r] = olen;
+							 t.r_crc[r] = crc;
+							 t.r_plen[r] = plen;
+							 t.r_cidx[r] = comp ? nc++ : 0xffffffffu;
+							 ++nd;
+						 });
+		t.nd[i] = nd;
+		t.nc[i] = nc;
+		t.walk_key[i] = key;
+		t.walk_out[i] = out;
+		t.verify_key[i] = kNone;
+	}
+}
+
+// One warp per stream: its region's records into the contiguous tables at the scanned bases, with the stream index and
+// absolute source / destination offsets.  Thread 0 also stores the batch totals next to each other for the read-back.
+__global__ void __launch_bounds__(256) framed_batch_compact_kernel(uint32_t n_streams, struct csb_framed_batch_rtable t)
+{
+	const uint32_t lane = threadIdx.x & 31u;
+	if (blockIdx.x == 0 && threadIdx.x == 0) {
+		t.totals[0] = t.d_base[n_streams];
+		t.totals[1] = t.c_base[n_streams];
+	}
+	const uint32_t warps = (gridDim.x * blockDim.x) >> 5;
+	for (uint32_t i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < n_streams; i += warps) {
+		const uint32_t nd = t.nd[i];
+		const uint64_t reg = t.s_reg[i], db = t.d_base[i], cb = t.c_base[i], so = t.s_src[i], doff = t.s_dst[i];
+		for (uint32_t j = lane; j < nd; j += 32) {
+			const uint64_t r = reg + j, k = db + j;
+			const uint64_t pos = so + t.r_pos[r], o = doff + t.r_out[r];
+			const uint32_t ci = t.r_cidx[r];
+			t.pos[k] = pos;
+			t.out_off[k] = o;
+			t.out_len[k] = t.r_len[r];
+			t.crc[k] = t.r_crc[r];
+			t.stream[k] = i;
+			if (ci != 0xffffffffu) {
+				const uint64_t c = cb + ci;
+				t.cidx[k] = (uint32_t)c;
+				t.c_pos[c] = pos;
+				t.c_len[c] = t.r_plen[r];
+				t.c_out_off[c] = o;
+			} else {
+				t.cidx[k] = 0xffffffffu;
+			}
+		}
+	}
+}
+
+// One warp per data chunk of the batch: framed_verify_kernel's checks; the failure key, relative to the chunk's
+// stream, goes to that stream's verify_key only.
+__global__ void __launch_bounds__(256) framed_batch_verify_kernel(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst,
+								  struct csb_framed_batch_rtable t)
+{
+	__shared__ CrcTables T;
+	load_crc_tables(T);
+	const uint64_t nd = t.totals[0];
+	const uint32_t warps = (gridDim.x * blockDim.x) >> 5;
+	for (uint64_t i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < nd; i += warps) {
+		const uint64_t pos = t.pos[i];
+		const uint32_t olen = t.out_len[i], j = t.cidx[i], st = t.stream[i];
+		uint8_t *o = dst + t.out_off[i];
+		const uint64_t rel = pos - t.s_src[st];
+		uint64_t key = kNone;
+		uint32_t c;
+		if (j != 0xffffffffu) {
+			if (t.c_status[j] != 0 || t.c_produced[j] != olen) {
+				key = rel * 4 + kClassMalformed;
+				c = 0;
+			} else {
+				c = warp_crc32c(T, o, olen);
+			}
+		} else {
+			const uint8_t *s = src + pos + 8;
+			warp_copy(o, s, olen);
+			c = warp_crc32c(T, s, olen);
+		}
+		if (key == kNone && c != t.crc[i])
+			key = rel * 4 + kClassChecksum;
+		if ((threadIdx.x & 31u) == 0 && key != kNone)
+			atomicMin(reinterpret_cast<unsigned long long *>(&t.verify_key[st]), (unsigned long long)key);
+	}
+}
+
+// One thread per stream: its result from the smaller of its walk and verify keys, as framed_finish_kernel, with the
+// binary search confined to the stream's own range of the compacted table.
+__global__ void __launch_bounds__(128) framed_batch_finish_kernel(uint32_t n_streams, struct csb_framed_batch_rtable t,
+								  uint64_t *__restrict__ out_length,
+								  int32_t *__restrict__ status,
+								  uint64_t *__restrict__ failed_offset)
+{
+	const uint32_t threads = gridDim.x * blockDim.x;
+	for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_streams; i += threads) {
+		const uint64_t wk = t.walk_key[i], vk = t.verify_key[i];
+		const uint64_t key = wk < vk ? wk : vk;
+		if (key == kNone) {
+			status[i] = 0;
+			out_length[i] = t.walk_out[i];
+			continue;
+		}
+		const uint64_t pos = key >> 2;
+		const uint32_t cls = (uint32_t)(key & 3u);
+		uint64_t produced = t.walk_out[i];  // a walk failure: every data chunk recorded lies before it
+		if (key != wk) {
+			const uint64_t at = t.s_src[i] + pos;
+			uint64_t lo = t.d_base[i], hi = lo + t.nd[i];  // the data chunk at `pos` (positions ascend)
+			while (hi - lo > 1) {
+				const uint64_t mid = (lo + hi) / 2;
+				if (t.pos[mid] <= at)
+					lo = mid;
+				else
+					hi = mid;
+			}
+			produced = t.out_off[lo] - t.s_dst[i];
+		}
+		status[i] = cls == kClassMalformed ? -5 : (cls == kClassOutput ? -2 : -102);
+		out_length[i] = produced;
+		if (failed_offset)
+			failed_offset[i] = pos;
+	}
+}
+
 static int grid_for(uint32_t units, int per_cta, int sm_count)
 {
 	long ctas = ((long)units + per_cta - 1) / per_cta;
@@ -443,6 +669,85 @@ extern "C" int csb_launch_framed_verify(const uint8_t *src, uint8_t *dst, uint32
 			return e;
 	}
 	framed_finish_kernel<<<1, 1, 0, s>>>(*t, out_length, status, failed_offset);
+	count_launch();
+	return (int)cudaGetLastError();
+}
+
+extern "C" int csb_launch_framed_batch_crc(const uint8_t *in, uint32_t n_chunks, const struct csb_framed_batch_wtable *t,
+					   csb_stream_t s)
+{
+	DeviceInfo di;
+	int e = device_info(&di);
+	if (e)
+		return e;
+	framed_batch_crc_kernel<<<grid_for(n_chunks, 8, di.sm_count), 256, 0, s>>>(in, n_chunks, *t);
+	count_launch();
+	return (int)cudaGetLastError();
+}
+
+extern "C" int csb_launch_framed_batch_write(const uint8_t *in, uint32_t n_chunks, uint32_t n_streams, const uint8_t *slots,
+					     uint64_t slot_stride, const struct csb_framed_batch_wtable *t, uint8_t *out,
+					     uint64_t *out_length, csb_stream_t s)
+{
+	DeviceInfo di;
+	int e = device_info(&di);
+	if (e)
+		return e;
+	const uint32_t units = n_chunks > n_streams / 32 ? n_chunks : n_streams / 32;
+	framed_batch_write_kernel<<<grid_for(units, 8, di.sm_count), 256, 0, s>>>(in, n_chunks, n_streams, slots, slot_stride,
+										    *t, out, out_length);
+	count_launch();
+	return (int)cudaGetLastError();
+}
+
+// one thread per stream: small CTAs, so that few streams still spread over the SMs
+static int grid_per_stream(uint32_t n_streams, int sm_count)
+{
+	long ctas = ((long)n_streams + 127) / 128;
+	if (ctas > (long)sm_count * 16)
+		ctas = (long)sm_count * 16;
+	return ctas < 1 ? 1 : (int)ctas;
+}
+
+extern "C" int csb_launch_framed_batch_walk(const uint8_t *src, uint32_t n_streams, const struct csb_framed_batch_rtable *t,
+					    uint64_t *length, int32_t *status, csb_stream_t s)
+{
+	DeviceInfo di;
+	int e = device_info(&di);
+	if (e)
+		return e;
+	framed_batch_walk_kernel<<<grid_per_stream(n_streams, di.sm_count), 128, 0, s>>>(src, n_streams, *t, length, status);
+	count_launch();
+	return (int)cudaGetLastError();
+}
+
+extern "C" int csb_launch_framed_batch_compact(uint32_t n_streams, const struct csb_framed_batch_rtable *t, csb_stream_t s)
+{
+	DeviceInfo di;
+	int e = device_info(&di);
+	if (e)
+		return e;
+	framed_batch_compact_kernel<<<grid_for(n_streams, 8, di.sm_count), 256, 0, s>>>(n_streams, *t);
+	count_launch();
+	return (int)cudaGetLastError();
+}
+
+extern "C" int csb_launch_framed_batch_verify(const uint8_t *src, uint8_t *dst, uint32_t n_data, uint32_t n_streams,
+					      const struct csb_framed_batch_rtable *t, uint64_t *out_length, int32_t *status,
+					      uint64_t *failed_offset, csb_stream_t s)
+{
+	DeviceInfo di;
+	int e = device_info(&di);
+	if (e)
+		return e;
+	if (n_data) {
+		framed_batch_verify_kernel<<<grid_for(n_data, 8, di.sm_count), 256, 0, s>>>(src, dst, *t);
+		count_launch();
+		if ((e = (int)cudaGetLastError()))
+			return e;
+	}
+	framed_batch_finish_kernel<<<grid_per_stream(n_streams, di.sm_count), 128, 0, s>>>(n_streams, *t, out_length, status,
+											     failed_offset);
 	count_launch();
 	return (int)cudaGetLastError();
 }

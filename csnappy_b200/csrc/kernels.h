@@ -109,6 +109,48 @@ int csb_launch_framed_walk(const uint8_t *src, uint64_t len, uint64_t cap, const
 int csb_launch_framed_verify(const uint8_t *src, uint8_t *dst, uint32_t n_data, const struct csb_framed_table *t,
 			     uint64_t *out_length, int32_t *status, uint64_t *failed_offset, csb_stream_t s);
 
+/* Many framed streams in one call.  Writer tables, laid out by the host: per 32 KiB fragment (compress input), per
+ * 65536-byte chunk and per stream; crc / rec / off are written on the device. */
+struct csb_framed_batch_wtable {
+	const uint32_t *flen;	  /* compressed size per fragment (compress output) */
+	const uint64_t *c_in;	  /* per chunk: absolute input offset */
+	const uint32_t *c_len;	  /* per chunk: bytes, 1..65536 */
+	const uint32_t *c_stream; /* per chunk: its stream */
+	const uint32_t *c_frag;	  /* per chunk: its first fragment (a second one follows when c_len > 32768) */
+	uint32_t *crc, *rec;	  /* per chunk: masked CRC, record size */
+	const uint64_t *off;	  /* per chunk: scanned record offset; off[n_chunks] = total */
+	const uint64_t *s_out;	  /* per stream: absolute output slot */
+	const uint32_t *s_first;  /* per stream: first chunk; s_first[n_streams] = n_chunks */
+};
+/* Reader tables.  The walk of stream i writes its data chunks into its own region [s_reg[i], s_reg[i] + s_len[i] / 8 + 1)
+ * of the r_* tables with stream-relative positions; the compaction copies them into the contiguous d_* / c_* tables
+ * (stream order, absolute offsets) at the scanned counts d_base / c_base. */
+struct csb_framed_batch_rtable {
+	const uint64_t *s_src, *s_len, *s_dst, *s_cap, *s_reg; /* per stream, from the host */
+	uint32_t *nd, *nc;				       /* per stream: data / compressed chunks recorded */
+	uint64_t *walk_key, *walk_out, *verify_key;	       /* per stream, as csb_framed_result */
+	uint64_t *d_base, *c_base;			       /* scans of nd / nc, n_streams + 1 entries */
+	uint64_t *totals;				       /* [0] data chunks, [1] compressed chunks of the batch */
+	uint64_t *r_pos, *r_out;			       /* region tables: relative position / output offset */
+	uint32_t *r_len, *r_crc, *r_cidx, *r_plen;	       /* r_cidx: stream-local compressed index, ~0 stored */
+	uint64_t *pos, *out_off;			       /* compacted data chunks: absolute src / dst offsets */
+	uint32_t *out_len, *crc, *cidx, *stream;
+	uint64_t *c_pos, *c_out_off; /* compacted compressed chunks: decoder input src + 8 + c_pos[j], c_len[j] bytes */
+	uint32_t *c_len, *c_produced;
+	int32_t *c_status;
+};
+int csb_launch_framed_batch_crc(const uint8_t *in, uint32_t n_chunks, const struct csb_framed_batch_wtable *t, csb_stream_t s);
+int csb_launch_framed_batch_write(const uint8_t *in, uint32_t n_chunks, uint32_t n_streams, const uint8_t *slots,
+				  uint64_t slot_stride, const struct csb_framed_batch_wtable *t, uint8_t *out,
+				  uint64_t *out_length, csb_stream_t s);
+/* length != NULL: the decompressed_length walk (unbounded capacity, no table writes) into length[i] / status[i] */
+int csb_launch_framed_batch_walk(const uint8_t *src, uint32_t n_streams, const struct csb_framed_batch_rtable *t,
+				 uint64_t *length, int32_t *status, csb_stream_t s);
+int csb_launch_framed_batch_compact(uint32_t n_streams, const struct csb_framed_batch_rtable *t, csb_stream_t s);
+int csb_launch_framed_batch_verify(const uint8_t *src, uint8_t *dst, uint32_t n_data, uint32_t n_streams,
+				   const struct csb_framed_batch_rtable *t, uint64_t *out_length, int32_t *status,
+				   uint64_t *failed_offset, csb_stream_t s);
+
 #ifdef __cplusplus
 }
 #endif

@@ -263,6 +263,55 @@ int csnappy_framed_compress_host(const void *h_in, uint64_t input_length, void *
 int csnappy_framed_decompress_host(const void *h_src, uint64_t src_length, void *h_dst, uint64_t out_capacity,
 				   uint64_t *out_length, uint64_t *failed_offset);
 
+/*
+ * MANY framed streams in one call, device resident, asynchronous on `stream`.  A batch call means exactly n_streams
+ * independent single calls: every result below is what csnappy_framed_compress / csnappy_framed_decompress returns
+ * for that stream alone, and one stream's content never affects another stream's result.  Stream i is
+ * d_in + h_in_off[i] (d_src + h_src_off[i]), h_in_len[i] (h_src_len[i]) bytes, any byte offset.  The offsets, lengths
+ * and capacities are HOST arrays: the host lays out the chunk tables and sizes the launches.  The launch count does
+ * not grow with n_streams.
+ *
+ * Writer (csnappy_framed_batch_compress):
+ *   output slot i is d_out + h_out_off[i]; h_out_off == NULL: slot i starts at the sum of
+ *   csnappy_framed_max_length(h_in_len[j]) for j < i.  Every slot [start, start + csnappy_framed_max_length(h_in_len[i]))
+ *   must end at or before out_capacity (else CSNAPPY_E_BAD_ARG); slots must not overlap (not checked).
+ *   Slot i receives exactly the bytes csnappy_framed_compress(stream i, wm) writes, d_out_len[i] <- that length (an
+ *   empty stream: the 10-byte identifier only).  Bytes outside [slot i, slot i + d_out_len[i]) are not written.
+ * Reader (csnappy_framed_batch_decompress):
+ *   d_status[i], d_out_len[i], d_failed_offset[i] and d_dst[h_dst_off[i], + d_out_len[i]) are exactly what
+ *   csnappy_framed_decompress returns for stream i with out_capacity h_dst_cap[i] (0 / -2 / -5 / -102, which failing
+ *   chunk wins, the valid prefix).  d_failed_offset[i] is measured from the start of stream i and written only when
+ *   stream i fails; d_failed_offset may be NULL.  Nothing is written at or past h_dst_off[i] + h_dst_cap[i].  The
+ *   call synchronises with `stream` once (the chunk totals of the batch size the launches), whatever n_streams is.
+ * Decompressed length (csnappy_framed_batch_decompressed_length): a framed stream does not carry its total length.
+ *   d_length[i] <- the sum of the data lengths its chunk headers declare (the varint of a 0x00 chunk, the body length
+ *   minus 4 of a 0x01 chunk) up to the first failure the chunk walk can detect; d_status[i] <- -5 if there is such a
+ *   failure, else 0.  Decoding stream i with capacity d_length[i] never returns CSNAPPY_E_OUTPUT_INSUF.  No workspace
+ *   and no synchronisation: the 16 bytes per stream of offsets and lengths go to a stream-ordered allocation
+ *   (cudaMallocAsync / cudaFreeAsync on `stream`, from the device's default memory pool) for the duration of the walk.
+ * Limits: per stream those of the single calls (input at most (2^32 - 2) * 32768 bytes, source at most 2^35 bytes);
+ *   per batch the fragments of the writer and the chunk table entries of the reader (sum of h_src_len[i] / 8 + 1) each
+ *   at most 2^32 - 1.  The workspace functions return UINT64_MAX for a batch beyond them.
+ * Returns 0 (n_streams == 0 included), CSNAPPY_E_DEVICE or CSNAPPY_E_BAD_ARG for the call as a whole; a refused
+ * argument (wm outside 9..16, a stream or batch beyond the limits, a slot past out_capacity, a short workspace, a NULL
+ * buffer) returns CSNAPPY_E_BAD_ARG before any device work.  d_workspace stays untouched until the work on `stream`
+ * has finished.
+ */
+uint64_t csnappy_framed_batch_compress_workspace(const uint64_t *h_in_len, uint32_t n_streams);
+int csnappy_framed_batch_compress(const void *d_in, const uint64_t *h_in_off, const uint64_t *h_in_len,
+				  uint32_t n_streams, void *d_out, const uint64_t *h_out_off,
+				  uint64_t out_capacity, uint64_t *d_out_len, int workmem_bytes_power_of_two,
+				  void *d_workspace, uint64_t workspace_bytes, void *stream);
+uint64_t csnappy_framed_batch_decompress_workspace(const uint64_t *h_src_len, uint32_t n_streams);
+int csnappy_framed_batch_decompress(const void *d_src, const uint64_t *h_src_off, const uint64_t *h_src_len,
+				    uint32_t n_streams, void *d_dst, const uint64_t *h_dst_off,
+				    const uint64_t *h_dst_cap, uint64_t *d_out_len, int32_t *d_status,
+				    uint64_t *d_failed_offset, void *d_workspace, uint64_t workspace_bytes,
+				    void *stream);
+int csnappy_framed_batch_decompressed_length(const void *d_src, const uint64_t *h_src_off,
+					     const uint64_t *h_src_len, uint32_t n_streams,
+					     uint64_t *d_length, int32_t *d_status, void *stream);
+
 /* Masked CRC-32C of each 65536-byte chunk of d_in[0, length) (the last one shorter) -> d_crc[ceil(length / 65536)];
  * the framing format's checksum, on the device, asynchronous on `stream`. */
 int csnappy_framed_crc32c(const void *d_in, uint64_t length, uint32_t *d_crc, void *stream);

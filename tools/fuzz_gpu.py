@@ -7,7 +7,9 @@ leg gets random streams of every tag form (tests/streams.py), which the compress
 writes a page container of random page size and length, corrupts its index and payload at random and compares the
 reader with the restated reader (tests/containers.py).  The framed leg round-trips a random buffer through the framing
 format, compares the stream with the restated writer, corrupts it at random and compares the reader with the restated
-reader (tests/framed.py).
+reader (tests/framed.py).  The batched-framed leg writes several random buffers in one csnappy_framed_batch_compress
+call, corrupts some of the streams, and reads valid and hostile streams together in one csnappy_framed_batch_decompress
+call, each against the restated writer and reader.
 
     python tools/fuzz_gpu.py [seconds] [seed]
 """
@@ -32,7 +34,7 @@ seed = int(sys.argv[2]) if len(sys.argv) > 2 else 20261017
 chk = oracle.best()
 rng = np.random.default_rng(seed)
 t0 = time.time()
-rounds = blocks = streams = pages_read = framed_streams = 0
+rounds = blocks = streams = pages_read = framed_streams = batch_framed = 0
 while time.time() - t0 < budget:
     size = int(rng.choice([17, 64, 300, 1000, 4096, 4096, 4096, 5000, 16384, 32768]))
     wm = int(rng.integers(9, 17))
@@ -146,6 +148,27 @@ while time.time() - t0 < budget:
     rc, out, bad = cs.api.framed_decompress(bytes(broken), cap)
     assert (rc, len(out), bad) == want.key() and out == want.data, ("framed read", len(data), want.key(), (rc, len(out), bad))
     framed_streams += 1
+    # batched framed: valid and hostile streams mixed in one call, every one against the restatement
+    bufs = [containers.mixed_bytes(int(rng.integers(1 << 30)), int(rng.choice([0, int(rng.integers(0, 300)),
+                                                                               int(rng.integers(0, 3 * framed.CHUNK))])),
+                                   scale=int(rng.integers(64, 70000))) for _ in range(int(rng.integers(1, 12)))]
+    zs = cs.api.framed_batch_compress(bufs, wm)
+    assert zs == [framed.write_framed(b, wm) for b in bufs], ("framed batch write", wm, [len(b) for b in bufs])
+    hostile, caps = [], []
+    for z, b in zip(zs, bufs):
+        z = bytearray(z)
+        if rng.random() < 0.5 and z:
+            for _ in range(int(rng.integers(1, 4))):
+                z[int(rng.integers(0, len(z)))] ^= 1 << int(rng.integers(0, 8))
+        if rng.random() < 0.2:
+            z = z[: int(rng.integers(0, len(z) + 1))]
+        hostile.append(bytes(z))
+        caps.append(len(b) - int(rng.integers(0, 2)) * int(rng.integers(0, len(b) + 1)))
+    got = cs.api.framed_batch_decompress(hostile, caps)
+    for z, c, g in zip(hostile, caps, got):
+        want = framed.read_framed(z, c)
+        assert (g[0], len(g[1]), g[2]) == want.key() and g[1] == want.data, ("framed batch read", want.key(), g[0], len(g[1]), g[2])
+    batch_framed += len(bufs)
     rounds += 1
 cs.set_tuning("compress_lanes", 0)
 cs.set_tuning("decompress_lanes", 0)
@@ -153,4 +176,5 @@ cs.set_tuning("compress_stage_input", 0)
 cs.set_tuning("decompress_stage_input", 0)
 print(f"fuzz ok: {rounds} rounds, {blocks} blocks compressed byte-identically, {streams} streams decoded with identical results, "
       f"{pages_read} container pages written and read as restated, "
-      f"{framed_streams} framed streams written, corrupted and read as restated in {time.time() - t0:.0f} s")
+      f"{framed_streams} framed streams written, corrupted and read as restated, "
+      f"{batch_framed} streams through the batched framed calls in {time.time() - t0:.0f} s")
