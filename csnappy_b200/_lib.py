@@ -39,6 +39,13 @@ def _declare(L):
         "csnappy_batch_compress": (i, [vp, vp, u64, vp, u32, u32, vp, u64, vp, i, vp, u64, vp]),
         "csnappy_bc_compress_host_multi": (i, [vp, u64, u32, vp, u64, C.POINTER(C.c_uint64), i, vp, i]),
         "csnappy_bc_decompress_host_multi": (i, [vp, u64, u32, vp, u64, C.POINTER(C.c_uint64), _u32p, vp, i]),
+        "csnappy_bc_compress_workspace": (u64, [u64, u32]),
+        "csnappy_bc_compress": (i, [vp, u64, u32, vp, u64, vp, i, vp, u64, vp]),
+        "csnappy_bc_index": (i, [vp, u64, u32, vp, u64, _u32p, vp]),
+        "csnappy_bc_decompress_pages_workspace": (u64, [u32]),
+        "csnappy_bc_decompress_pages": (i, [vp, u64, u32, vp, u32, vp, u32, vp, u64, vp, vp, vp, u64, vp]),
+        "csnappy_bc_decompress_workspace": (u64, [u64, u32, u64]),
+        "csnappy_bc_decompress": (i, [vp, u64, u32, vp, u64, vp, vp, vp, vp, u64, vp]),
         "csnappy_stream_decompress_workspace": (u64, [u32, u32]),
         "csnappy_stream_decompress": (i, [vp, u32, vp, u32, vp, vp, vp, u64, vp]),
         "csnappy_framed_max_length": (u64, [u64]),

@@ -12,6 +12,9 @@ Device-resident batches (torch CUDA tensors, asynchronous on the current stream)
     batch_compress_fragments, batch_decompress, batch_pack
 Host-buffer batches (numpy / pinned torch tensors, synchronous, pipelined H2D/D2H):
     batch_compress_fragments_host, batch_decompress_host
+block_compressor page container: bc_compress_host, bc_decompress_host (host buffers); bc_compress_device,
+    bc_index_device, bc_decompress_pages_device (random page reads), bc_decompress_device (CUDA tensors, current
+    stream)
 Snappy framing format (64 KiB chunks with masked CRC-32C):
     framed_compress, framed_decompress (host bytes); framed_compress_device, framed_decompress_device,
     framed_crc32c_device (CUDA tensors, current stream); many streams in one call: framed_batch_compress,
@@ -254,6 +257,120 @@ def bc_decompress_host_multi(h_container, container_length: int, h_out, page_siz
     if rc in (CSNAPPY_E_DEVICE, CSNAPPY_E_BAD_ARG):
         _check(rc, "csnappy_bc_decompress_host_multi")
     return rc, olen.value, (bad.value if rc != 0 and bad.value != 0xFFFFFFFF else None)
+
+
+BC_NO_PAGE = 2**64 - 1  # index entry of a page outside the decodable prefix (read as -1 from an int64 tensor)
+
+
+def _ws(nbytes: int, device):
+    """A workspace tensor; a workspace function's UINT64_MAX (arguments beyond the limits) is left to the C call to
+    refuse."""
+    import torch
+
+    return torch.empty(max(nbytes, 1) if nbytes < 1 << 62 else 1, dtype=torch.uint8, device=device)
+
+
+def bc_compress_device(d_in, input_length: int | None = None, wm: int = 13, page_size: int = 4096, *, out=None,
+                       out_length=None, workspace=None):
+    """Page container of a uint8 CUDA tensor written on the device, asynchronous on the current stream; the same bytes
+    as bc_compress_host.  Returns (container uint8 [bc_max_container_length(n)], length int64 [1]) CUDA tensors."""
+    import torch
+
+    n = d_in.numel() if input_length is None else input_length
+    if out is None:
+        out = torch.empty(max(bc_max_container_length(n, page_size), 1), dtype=torch.uint8, device=d_in.device)
+    if out_length is None:
+        out_length = torch.empty(1, dtype=torch.int64, device=d_in.device)
+    if workspace is None:
+        workspace = _ws(lib().csnappy_bc_compress_workspace(n, page_size), d_in.device)
+    rc = lib().csnappy_bc_compress(_ptr(d_in), n, page_size, _ptr(out), out.numel(), _ptr(out_length), wm,
+                                   _ptr(workspace), workspace.numel(), _stream_ptr())
+    _check(rc, "csnappy_bc_compress")
+    return out, out_length  # the workspace is freed in stream order, as in framed_compress_device
+
+
+def bc_index_device(d_container, container_length: int | None = None, page_size: int = 4096, *, index=None):
+    """Payload offset of every page of a container in device memory (the call reads the page count back).
+    Returns (rc, index int64 CUDA tensor, nr_pages): rc 0, or CSNAPPY_E_DATA_MALFORMED for a container shorter than
+    its index.  index[i] is -1 (BC_NO_PAGE) from the first malformed entry on.  Without `index`, one is allocated for
+    the page count (a first call reads the count)."""
+    import torch
+
+    n = d_container.numel() if container_length is None else container_length
+    nr = C.c_uint32(0)
+    if index is None:
+        rc = lib().csnappy_bc_index(_ptr(d_container), n, page_size, None, 0, C.byref(nr), _stream_ptr())
+        if rc == CSNAPPY_E_BAD_ARG and nr.value:  # the count was read: size the index and ask again
+            rc = 0
+        if rc == CSNAPPY_E_DATA_MALFORMED:
+            return rc, torch.empty(0, dtype=torch.int64, device=d_container.device), nr.value
+        _check(rc, "csnappy_bc_index")
+        index = torch.empty(max(nr.value, 1), dtype=torch.int64, device=d_container.device)
+    rc = lib().csnappy_bc_index(_ptr(d_container), n, page_size, _ptr(index), index.numel(), C.byref(nr), _stream_ptr())
+    if rc != CSNAPPY_E_DATA_MALFORMED:
+        _check(rc, "csnappy_bc_index")
+    return rc, index, nr.value
+
+
+def bc_decompress_pages_device(d_container, index, nr_pages: int, pages, page_size: int = 4096,
+                               container_length: int | None = None, *, out=None, out_stride: int | None = None,
+                               out_len=None, status=None, workspace=None):
+    """Decode the pages numbered by `pages` (int32 CUDA tensor, read as uint32) of a container in device memory, with
+    `index` / `nr_pages` from bc_index_device; request k goes to out[k * out_stride, + page_size).  Asynchronous on
+    the current stream.  Returns (out uint8, out_len int32, status int32) CUDA tensors; status per request: 0, the
+    page's decode result, CSNAPPY_E_DATA_MALFORMED (page outside the decodable prefix) or CSNAPPY_E_BAD_ARG (page
+    number >= nr_pages)."""
+    import torch
+
+    n = pages.numel()
+    size = d_container.numel() if container_length is None else container_length
+    out_stride = page_size if out_stride is None else out_stride
+    dev = d_container.device
+    if out is None:
+        out = torch.empty(max(n * out_stride, 1), dtype=torch.uint8, device=dev)
+    if out_len is None:
+        out_len = torch.empty(max(n, 1), dtype=torch.int32, device=dev)
+    if status is None:
+        status = torch.empty(max(n, 1), dtype=torch.int32, device=dev)
+    if workspace is None:
+        workspace = _ws(lib().csnappy_bc_decompress_pages_workspace(n), dev)
+    rc = lib().csnappy_bc_decompress_pages(_ptr(d_container), size, page_size, _ptr(index), nr_pages, _ptr(pages), n,
+                                           _ptr(out), out_stride, _ptr(out_len), _ptr(status), _ptr(workspace),
+                                           workspace.numel(), _stream_ptr())
+    _check(rc, "csnappy_bc_decompress_pages")
+    return out, out_len, status
+
+
+def bc_decompress_device(d_container, container_length: int | None = None, page_size: int = 4096,
+                         out_capacity: int | None = None, *, out=None, result=None, workspace=None):
+    """Whole container in device memory -> its pages, page i at out[i * page_size] (the call reads the page count
+    back, then enqueues the rest on the current stream).  out_capacity None: out's size, or nr_pages * page_size.
+    Returns (out uint8, result int64 [3] = [out_length, rc, failed_page]) CUDA tensors with the values
+    bc_decompress_host returns; result[2] is written only when a page fails (default prefilled with -1)."""
+    import torch
+
+    n = d_container.numel() if container_length is None else container_length
+    dev = d_container.device
+    if out_capacity is None:
+        if out is not None:
+            out_capacity = out.numel()
+        else:
+            out_capacity = (int.from_bytes(d_container[:4].cpu().numpy().tobytes(), "little") if n >= 4 else 0) * page_size
+    if out is None:
+        out = torch.empty(max(out_capacity, 1), dtype=torch.uint8, device=dev)
+    if result is None:
+        result = torch.full((3,), -1, dtype=torch.int64, device=dev)
+    words = torch.full((2,), -1, dtype=torch.int32, device=dev)  # status, failed page (u32)
+    if workspace is None:
+        workspace = _ws(lib().csnappy_bc_decompress_workspace(n, page_size, out_capacity), dev)
+    rc = lib().csnappy_bc_decompress(_ptr(d_container), n, page_size, _ptr(out), out_capacity, result.data_ptr(),
+                                     words.data_ptr(), words.data_ptr() + 4, _ptr(workspace), workspace.numel(),
+                                     _stream_ptr())
+    _check(rc, "csnappy_bc_decompress")
+    result[1:2].copy_(words[:1])
+    failed = words[1:2].to(torch.int64) & 0xFFFFFFFF
+    result[2:3].copy_(torch.where(words[1:2] == -1, result[2:3], failed))
+    return out, result
 
 
 def batch_compress(d_in, in_off, in_len, wm: int, *, out_stride: int | None = None):

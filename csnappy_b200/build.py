@@ -23,7 +23,7 @@ CUDA_HOME = os.environ.get("CUDA_HOME", "/usr/local/cuda")
 NVCC = shutil.which("nvcc") or os.path.join(CUDA_HOME, "bin", "nvcc")
 
 CU = ["compress_kernel.cu", "decompress_kernel.cu", "decompress_lane_kernel.cu", "stream_kernel.cu", "pack_kernel.cu",
-      "framed_kernel.cu"]
+      "framed_kernel.cu", "bc_kernel.cu"]
 C = ["csnappy_shim.c"]
 HEADERS = [os.path.join(CSRC, h) for h in ("kernels.h", "device_common.cuh")] + [
     os.path.join(HERE, "..", "include", h) for h in ("csnappy.h", "csnappy_batch.h")

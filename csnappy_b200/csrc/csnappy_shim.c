@@ -1814,6 +1814,284 @@ int csnappy_bc_decompress_host_multi(const void *h_container, uint64_t container
 	return bc_decompress(h_container, container_length, page_size, h_out, out_capacity, out_length, failed_page, list, G);
 }
 
+/* ---- the same container on DEVICE buffers (csnappy_bc_compress / _index / _decompress_pages / _decompress) ---------
+ * Writer: one compress launch over every page (total_len clips the short last page), the stored-page rule
+ * (csb_launch_clamp), the grid-wide index scan for the payload offsets, the gather of fragments and stored pages to
+ * their offsets, and the header and index at d_container (bc_kernel.cu; any alignment).
+ * Readers: the page count is read back (one synchronisation); the index scan gives each page's payload offset, or
+ * CSNAPPY_BC_NO_PAGE from the first malformed entry on.  A batch of page requests gathers (offset, length) per request
+ * and runs the batched decoder on those; the whole-container read runs the decoder on every page with the index as
+ * its offsets, and a finish step reduces the page results to the host reader's (status, out_length, failed_page). */
+#define BC_MAX_PAGES 0xffffffffull
+
+static uint64_t bc_pages_of(uint64_t input_length, uint32_t page) { return input_length / page + (input_length % page != 0); }
+
+static uint64_t bc_slot(uint32_t page) { return ((uint64_t)csnappy_max_compressed_length(page) + 15) & ~(uint64_t)15; }
+
+static int bc_page_size_ok(uint32_t page) { return page >= 1 && page <= CSB_FRAGMENT_MAX; }
+
+/* writer workspace: fragment slots | fragment sizes | stored-rule sizes | payload offsets | claim counter */
+static uint64_t bc_compress_layout(uint64_t nr, uint32_t page, uint64_t *o_len, uint64_t *o_clen, uint64_t *o_off,
+				   uint64_t *o_ctr)
+{
+	uint64_t p = al256(nr * bc_slot(page));
+	*o_len = p;
+	p = al256(p + nr * 4);
+	*o_clen = p;
+	p = al256(p + nr * 4);
+	*o_off = p;
+	p = al256(p + nr * 8);
+	*o_ctr = p;
+	return p + 256;
+}
+
+uint64_t csnappy_bc_compress_workspace(uint64_t input_length, uint32_t page_size)
+{
+	uint64_t nr, a, b, c, d;
+	if (!bc_page_size_ok(page_size))
+		return UINT64_MAX;
+	nr = bc_pages_of(input_length, page_size);
+	if (nr > BC_MAX_PAGES)
+		return UINT64_MAX;
+	return bc_compress_layout(nr, page_size, &a, &b, &c, &d);
+}
+
+int csnappy_bc_compress(const void *d_in, uint64_t input_length, uint32_t page_size, void *d_container,
+			uint64_t container_capacity, uint64_t *d_container_length, int workmem_bytes_power_of_two,
+			void *d_workspace, uint64_t workspace_bytes, void *stream)
+{
+	uint64_t nr, o_len, o_clen, o_off, o_ctr;
+	uint8_t *ws = (uint8_t *)d_workspace;
+	csb_stream_t s = (csb_stream_t)stream;
+	struct csb_compress_args a;
+	int e;
+	if (workmem_bytes_power_of_two < 9 || workmem_bytes_power_of_two > 16)
+		return set_err("workmem_bytes_power_of_two outside 9..16", 0);
+	if (!bc_page_size_ok(page_size))
+		return set_err("page_size outside 1..32768", 0);
+	nr = bc_pages_of(input_length, page_size);
+	if (nr > BC_MAX_PAGES)
+		return set_err("more than 2^32 - 1 pages", 0);
+	if (!d_container || !d_container_length || !d_workspace || (input_length && !d_in))
+		return set_err("null buffer", 0);
+	if (container_capacity < csnappy_bc_max_container_length(input_length, page_size))
+		return set_err("container_capacity smaller than csnappy_bc_max_container_length()", 0);
+	if (workspace_bytes < bc_compress_layout(nr, page_size, &o_len, &o_clen, &o_off, &o_ctr))
+		return set_err("workspace smaller than csnappy_bc_compress_workspace()", 0);
+	if (nr) {
+		fill_compress_args(&a);
+		a.in = (const uint8_t *)d_in;
+		a.in_stride = page_size;
+		a.uniform_len = page_size;
+		a.total_len = input_length;
+		a.n_blocks = (uint32_t)nr;
+		a.out = ws;
+		a.out_stride = bc_slot(page_size);
+		a.out_len = (uint32_t *)(ws + o_len);
+		a.wm = workmem_bytes_power_of_two;
+		a.counter = (uint32_t *)(ws + o_ctr);
+		if ((e = csb_launch_compress(&a, s)))
+			return set_err("compress launch", e);
+		if ((e = csb_launch_clamp((const uint32_t *)(ws + o_len), (uint32_t)nr, page_size, input_length,
+					  (uint32_t *)(ws + o_clen), s)))
+			return set_err("clamp launch", e);
+		/* every size is valid here: no bound, no room limit */
+		if ((e = csb_launch_bc_index(ws + o_clen, (uint32_t)nr, 0xffffffffu, 4 + 4 * nr, UINT64_MAX, 0,
+					     (uint64_t *)(ws + o_off), NULL, NULL, s)))
+			return set_err("index launch", e);
+		if ((e = csb_launch_gather(ws, bc_slot(page_size), (const uint32_t *)(ws + o_clen), (uint32_t)nr,
+					   (uint8_t *)d_container, (const uint64_t *)(ws + o_off), (const uint8_t *)d_in, page_size,
+					   input_length, (const uint32_t *)(ws + o_len), s)))
+			return set_err("gather launch", e);
+	}
+	e = csb_launch_bc_header((const uint32_t *)(ws + o_clen), (uint32_t)nr, (const uint64_t *)(ws + o_off),
+				 (uint8_t *)d_container, d_container_length, s);
+	return e ? set_err("header launch", e) : 0;
+}
+
+/* the page count at the container's start: the readers' one synchronisation */
+static int bc_read_count(const void *d_container, uint32_t *nr, cudaStream_t s)
+{
+	int e;
+	if ((e = (int)cudaMemcpyAsync(nr, d_container, 4, cudaMemcpyDeviceToHost, s)) || (e = (int)cudaStreamSynchronize(s)))
+		return set_err("D2H page count", e);
+	return 0;
+}
+
+int csnappy_bc_index(const void *d_container, uint64_t container_length, uint32_t page_size, uint64_t *d_index,
+		     uint64_t index_entries, uint32_t *nr_pages, void *stream)
+{
+	uint32_t nr = 0;
+	int e;
+	if (!bc_page_size_ok(page_size))
+		return set_err("page_size outside 1..32768", 0);
+	if (!d_container || !nr_pages || container_length < 4)
+		return set_err("container missing or shorter than its header", 0);
+	if (index_entries && !d_index)
+		return set_err("null buffer", 0);
+	if ((e = bc_read_count(d_container, &nr, (cudaStream_t)stream)))
+		return e;
+	*nr_pages = nr;
+	if (container_length < 4 + 4 * (uint64_t)nr)
+		return CSNAPPY_E_DATA_MALFORMED;
+	if (index_entries < nr)
+		return set_err("index_entries smaller than the page count", 0);
+	e = csb_launch_bc_index((const uint8_t *)d_container + 4, nr, csnappy_max_compressed_length(page_size),
+				4 + 4 * (uint64_t)nr, container_length - 4 - 4 * (uint64_t)nr, CSNAPPY_BC_NO_PAGE, d_index,
+				NULL, NULL, (csb_stream_t)stream);
+	return e ? set_err("index launch", e) : 0;
+}
+
+/* page reads workspace: decoder offsets | decoder lengths | request tags | claim counter */
+static uint64_t bc_pages_layout(uint64_t n, uint64_t *o_len, uint64_t *o_tag, uint64_t *o_ctr)
+{
+	uint64_t p = al256(n * 8);
+	*o_len = p;
+	p = al256(p + n * 4);
+	*o_tag = p;
+	p = al256(p + n * 4);
+	*o_ctr = p;
+	return p + 256;
+}
+
+uint64_t csnappy_bc_decompress_pages_workspace(uint32_t n_requests)
+{
+	uint64_t a, b, c;
+	return bc_pages_layout(n_requests, &a, &b, &c);
+}
+
+int csnappy_bc_decompress_pages(const void *d_container, uint64_t container_length, uint32_t page_size,
+				const uint64_t *d_index, uint32_t nr_pages, const uint32_t *d_pages, uint32_t n_requests,
+				void *d_out, uint64_t out_stride, uint32_t *d_out_len, int32_t *d_status,
+				void *d_workspace, uint64_t workspace_bytes, void *stream)
+{
+	uint64_t o_len, o_tag, o_ctr;
+	uint8_t *ws = (uint8_t *)d_workspace;
+	csb_stream_t s = (csb_stream_t)stream;
+	struct csb_decompress_args a;
+	int e;
+	if (!bc_page_size_ok(page_size))
+		return set_err("page_size outside 1..32768", 0);
+	if (out_stride < page_size)
+		return set_err("out_stride smaller than page_size", 0);
+	if (n_requests == 0)
+		return 0;
+	if (!d_container || !d_pages || !d_out || !d_out_len || !d_status || !d_workspace || (nr_pages && !d_index))
+		return set_err("null buffer", 0);
+	if (container_length < 4 + 4 * (uint64_t)nr_pages)
+		return set_err("container shorter than the index of nr_pages pages", 0);
+	if (workspace_bytes < bc_pages_layout(n_requests, &o_len, &o_tag, &o_ctr))
+		return set_err("workspace smaller than csnappy_bc_decompress_pages_workspace()", 0);
+	if ((e = csb_launch_bc_requests((const uint8_t *)d_container, container_length, csnappy_max_compressed_length(page_size),
+					d_index, nr_pages, d_pages, n_requests, (uint64_t *)ws, (uint32_t *)(ws + o_len),
+					(int32_t *)(ws + o_tag), s)))
+		return set_err("request launch", e);
+	fill_decompress_args(&a);
+	a.in = (const uint8_t *)d_container;
+	a.in_off = (const uint64_t *)ws;
+	a.in_len = (const uint32_t *)(ws + o_len);
+	a.n_blocks = n_requests;
+	a.out = (uint8_t *)d_out;
+	a.out_stride = out_stride;
+	a.uniform_cap = page_size;
+	a.out_len = d_out_len;
+	a.status = d_status;
+	a.flags = CSNAPPY_BATCH_RAW_IF_FULL;
+	a.counter = (uint32_t *)(ws + o_ctr);
+	if ((e = csb_launch_decompress(&a, s)))
+		return set_err("decompress launch", e);
+	e = csb_launch_bc_request_status((const int32_t *)(ws + o_tag), n_requests, d_out_len, d_status, s);
+	return e ? set_err("request status launch", e) : 0;
+}
+
+/* whole-container workspace, for the most pages a container of this length and an output of this capacity can take:
+ * index | decoder lengths | page out_len | page status | result words | claim counter */
+static uint64_t bc_decompress_layout(uint64_t container_length, uint32_t page, uint64_t out_capacity, uint64_t *o_len,
+				     uint64_t *o_olen, uint64_t *o_st, uint64_t *o_res, uint64_t *o_ctr)
+{
+	uint64_t n = container_length >= 4 ? (container_length - 4) / 4 : 0, p;
+	if (n > out_capacity / page)
+		n = out_capacity / page;
+	if (n > BC_MAX_PAGES)
+		n = BC_MAX_PAGES;
+	p = al256(n * 8);
+	*o_len = p;
+	p = al256(p + n * 4);
+	*o_olen = p;
+	p = al256(p + n * 4);
+	*o_st = p;
+	p = al256(p + n * 4);
+	*o_res = p;
+	p = al256(p + sizeof(struct csb_bc_result));
+	*o_ctr = p;
+	return p + 256;
+}
+
+uint64_t csnappy_bc_decompress_workspace(uint64_t container_length, uint32_t page_size, uint64_t out_capacity)
+{
+	uint64_t a, b, c, d, e;
+	if (!bc_page_size_ok(page_size))
+		return UINT64_MAX;
+	return bc_decompress_layout(container_length, page_size, out_capacity, &a, &b, &c, &d, &e);
+}
+
+int csnappy_bc_decompress(const void *d_container, uint64_t container_length, uint32_t page_size, void *d_out,
+			  uint64_t out_capacity, uint64_t *d_out_length, int32_t *d_status, uint32_t *d_failed_page,
+			  void *d_workspace, uint64_t workspace_bytes, void *stream)
+{
+	uint64_t o_len, o_olen, o_st, o_res, o_ctr;
+	uint8_t *ws = (uint8_t *)d_workspace;
+	cudaStream_t s = (cudaStream_t)stream;
+	struct csb_bc_result *res;
+	struct csb_decompress_args a;
+	uint32_t nr = 0;
+	int32_t hdr = 0;
+	int e;
+	if (!bc_page_size_ok(page_size))
+		return set_err("page_size outside 1..32768", 0);
+	if (!d_container || container_length < 4)
+		return set_err("container missing or shorter than its header", 0);
+	if (!d_out_length || !d_status || !d_workspace || (out_capacity && !d_out))
+		return set_err("null buffer", 0);
+	if (workspace_bytes < bc_decompress_layout(container_length, page_size, out_capacity, &o_len, &o_olen, &o_st, &o_res, &o_ctr))
+		return set_err("workspace smaller than csnappy_bc_decompress_workspace()", 0);
+	res = (struct csb_bc_result *)(ws + o_res);
+	if ((e = bc_read_count(d_container, &nr, s)))
+		return e;
+	if (container_length < 4 + 4 * (uint64_t)nr)
+		hdr = CSNAPPY_E_DATA_MALFORMED;
+	else if (out_capacity < (uint64_t)nr * page_size)
+		hdr = CSNAPPY_E_OUTPUT_INSUF;
+	if (!hdr && nr) {
+		if ((e = (int)cudaMemsetAsync(res, 0xff, offsetof(struct csb_bc_result, sum), s)) ||
+		    (e = (int)cudaMemsetAsync(&res->sum, 0, sizeof(res->sum), s)))
+			return set_err("result words", e);
+		/* pages behind the prefix decode an empty block at the container start: no output, and the finish step
+		 * does not count them */
+		if ((e = csb_launch_bc_index((const uint8_t *)d_container + 4, nr, csnappy_max_compressed_length(page_size),
+					     4 + 4 * (uint64_t)nr, container_length - 4 - 4 * (uint64_t)nr, 0, (uint64_t *)ws,
+					     (uint32_t *)(ws + o_len), &res->prefix, (csb_stream_t)s)))
+			return set_err("index launch", e);
+		fill_decompress_args(&a);
+		a.in = (const uint8_t *)d_container;
+		a.in_off = (const uint64_t *)ws;
+		a.in_len = (const uint32_t *)(ws + o_len);
+		a.n_blocks = nr;
+		a.out = (uint8_t *)d_out;
+		a.out_stride = page_size;
+		a.uniform_cap = page_size;
+		a.out_len = (uint32_t *)(ws + o_olen);
+		a.status = (int32_t *)(ws + o_st);
+		a.flags = CSNAPPY_BATCH_RAW_IF_FULL;
+		a.counter = (uint32_t *)(ws + o_ctr);
+		if ((e = csb_launch_decompress(&a, (csb_stream_t)s)))
+			return set_err("decompress launch", e);
+	}
+	e = csb_launch_bc_finish((const uint32_t *)(ws + o_olen), (const int32_t *)(ws + o_st), nr, hdr, res, d_out_length,
+				 d_status, d_failed_page, (csb_stream_t)s);
+	return e ? set_err("finish launch", e) : 0;
+}
+
 /* ---- Snappy framing format (include/csnappy_batch.h csnappy_framed_*; kernels in framed_kernel.cu) ------------------
  * Writer: ONE compress launch over the whole input as 32 KiB fragments (only the global last fragment is short, and it
  * gets csnappy_compress()'s short-chunk table rule), so fragments 2k and 2k+1 behind a varint are exactly

@@ -72,6 +72,13 @@ int csb_launch_pack_stored(const uint8_t *slots, uint64_t slot_stride, const uin
 			   const uint8_t *in, uint32_t page_len, uint64_t total_in, uint32_t *clen,
 			   uint8_t *packed, uint64_t *off, csb_stream_t s);
 int csb_launch_scan(const uint32_t *len, uint32_t n_blocks, uint64_t *off, csb_stream_t s);
+/* the two halves of csb_launch_pack_stored around its scan: clen[i] = min(len[i], input length of block i), and the
+ * gather of the slots (or, with raw, of the stored input blocks) to packed + off[i] */
+int csb_launch_clamp(const uint32_t *len, uint32_t n_blocks, uint32_t page_len, uint64_t total_in, uint32_t *clen,
+		     csb_stream_t s);
+int csb_launch_gather(const uint8_t *slots, uint64_t slot_stride, const uint32_t *len, uint32_t n_blocks, uint8_t *packed,
+		      const uint64_t *off, const uint8_t *raw, uint32_t page_len, uint64_t total_in, const uint32_t *slot_len,
+		      csb_stream_t s);
 /* batched csnappy_compress framing: header + fragments of every buffer into its output slot (pack_kernel.cu) */
 int csb_launch_frame(const uint8_t *slots, uint64_t slot_stride, const uint32_t *len, const uint64_t *off,
 		     const uint32_t *fbuf, const uint32_t *bfirst, const uint32_t *blen, uint32_t n_frag,
@@ -150,6 +157,34 @@ int csb_launch_framed_batch_compact(uint32_t n_streams, const struct csb_framed_
 int csb_launch_framed_batch_verify(const uint8_t *src, uint8_t *dst, uint32_t n_data, uint32_t n_streams,
 				   const struct csb_framed_batch_rtable *t, uint64_t *out_length, int32_t *status,
 				   uint64_t *failed_offset, csb_stream_t s);
+
+/* Page container on device buffers (bc_kernel.cu).
+ * Index scan of n u32 entries at ent (any alignment), grid-wide: index[i] = first_off + the sum of the entries before
+ * i while that sum plus entry i stays within room and no entry so far is above max_clen (the decodable prefix),
+ * bad_off for every later page.  len (optional): the entry inside the prefix, 0 behind it.  prefix (optional, set to
+ * 0xffffffff beforehand): the first page behind the prefix, left as it is when there is none.  index[] is the only
+ * memory the scan needs: each CTA's partial sum waits in the first word of its own range. */
+int csb_launch_bc_index(const uint8_t *ent, uint32_t n, uint32_t max_clen, uint64_t first_off, uint64_t room,
+			uint64_t bad_off, uint64_t *index, uint32_t *len, uint32_t *prefix, csb_stream_t s);
+/* [u32 n][u32 clen[n]] at cont (any alignment); *cont_length = index[n - 1] + clen[n - 1] (4 for n == 0) */
+int csb_launch_bc_header(const uint32_t *clen, uint32_t n, const uint64_t *index, uint8_t *cont, uint64_t *cont_length,
+			 csb_stream_t s);
+/* page requests -> decoder input in_off / in_len and tag (0, or the status of a request that is not decoded) */
+int csb_launch_bc_requests(const uint8_t *cont, uint64_t cont_length, uint32_t max_clen, const uint64_t *index,
+			   uint32_t nr, const uint32_t *pages, uint32_t n, uint64_t *in_off, uint32_t *in_len, int32_t *tag,
+			   csb_stream_t s);
+int csb_launch_bc_request_status(const int32_t *tag, uint32_t n, uint32_t *out_len, int32_t *status, csb_stream_t s);
+struct csb_bc_result {	/* device words of one whole-container read */
+	uint64_t key;	/* smallest (page << 32 | status) of a failed prefix page; set to ~0 beforehand */
+	uint32_t prefix; /* first page behind the decodable prefix; set to ~0 beforehand */
+	uint32_t pad;
+	uint64_t sum;	/* bytes produced by the prefix's good pages; set to 0 beforehand */
+};
+/* hdr_rc != 0 or nr == 0: *status = hdr_rc, *out_length = 0; else the reduction of out_len / status_pages over the
+ * prefix and the index error at its end into *status, *out_length and (on failure, when given) *failed_page */
+int csb_launch_bc_finish(const uint32_t *out_len, const int32_t *status_pages, uint32_t nr, int32_t hdr_rc,
+			 struct csb_bc_result *r, uint64_t *out_length, int32_t *status, uint32_t *failed_page,
+			 csb_stream_t s);
 
 #ifdef __cplusplus
 }

@@ -296,6 +296,41 @@ extern "C" int csb_launch_pack_stored(const uint8_t *slots, uint64_t slot_stride
 	return (int)cudaGetLastError();
 }
 
+extern "C" int csb_launch_clamp(const uint32_t *len, uint32_t n_blocks, uint32_t page_len, uint64_t total_in, uint32_t *clen,
+				csb_stream_t s)
+{
+	DeviceInfo di;
+	int e = device_info(&di);
+	if (e)
+		return e;
+	if (n_blocks == 0)
+		return 0;
+	long ctas = ((long)n_blocks + 255) / 256;
+	if (ctas > (long)di.sm_count * 4)
+		ctas = (long)di.sm_count * 4;
+	clamp_kernel<<<(int)ctas, 256, 0, s>>>(len, n_blocks, page_len, total_in, clen);
+	count_launch();
+	return (int)cudaGetLastError();
+}
+
+extern "C" int csb_launch_gather(const uint8_t *slots, uint64_t slot_stride, const uint32_t *len, uint32_t n_blocks,
+				 uint8_t *packed, const uint64_t *off, const uint8_t *raw, uint32_t page_len, uint64_t total_in,
+				 const uint32_t *slot_len, csb_stream_t s)
+{
+	DeviceInfo di;
+	int e = device_info(&di);
+	if (e)
+		return e;
+	if (n_blocks == 0)
+		return 0;
+	long ctas = ((long)n_blocks + 7) / 8;
+	if (ctas > (long)di.sm_count * 8)
+		ctas = (long)di.sm_count * 8;
+	gather_kernel<<<(int)ctas, 256, 0, s>>>(slots, slot_stride, len, n_blocks, packed, off, raw, page_len, total_in, slot_len);
+	count_launch();
+	return (int)cudaGetLastError();
+}
+
 extern "C" int csb_launch_scan(const uint32_t *len, uint32_t n_blocks, uint64_t *off, csb_stream_t s)
 {
 	scan_kernel<<<1, kScanThreads, 0, s>>>(len, n_blocks, off);

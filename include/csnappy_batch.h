@@ -21,8 +21,9 @@
  * reference, cl_tester.c:120-165) and >= capacity for decompression.
  * Fast paths engage when base, stride and offsets are multiples of 16.
  *
- * Every function returns 0, CSNAPPY_E_DEVICE or CSNAPPY_E_BAD_ARG (the framed and container readers also a
- * stream's decode result); per-block
+ * Every function returns 0, CSNAPPY_E_DEVICE or CSNAPPY_E_BAD_ARG (the framed and host container readers also a
+ * stream's decode result, csnappy_bc_index CSNAPPY_E_DATA_MALFORMED for a short index; the device container readers
+ * put theirs in device words); per-block
  * decoder results go to d_status[] / h_status[].
  */
 #ifndef CSNAPPY_B200_CSNAPPY_BATCH_H_
@@ -196,6 +197,62 @@ int csnappy_bc_decompress_host_multi(const void *h_container, uint64_t container
 				     uint32_t page_size, void *h_out, uint64_t out_capacity,
 				     uint64_t *out_length, uint32_t *failed_page,
 				     const int *devices, int n_devices);
+
+/*
+ * The same container on DEVICE buffers of the current device, asynchronous on `stream`: pages that already live in
+ * device memory are written into a container there, and a container in device memory (copied there with one
+ * cudaMemcpyAsync, or kept there compressed) is read there -- whole, or a batch of chosen pages.  Only the readers
+ * synchronise, once, to read the 4-byte page count; the launch count grows with neither the page count nor the
+ * number of requests.  Workspaces stay untouched until the work on `stream` has finished.  Every call returns 0,
+ * CSNAPPY_E_DEVICE or CSNAPPY_E_BAD_ARG (csnappy_bc_index also CSNAPPY_E_DATA_MALFORMED); a refused argument (page_size
+ * outside 1..32768, wm outside 9..16, more than 2^32 - 1 pages, a capacity below the bound, a short workspace, a NULL
+ * buffer) returns CSNAPPY_E_BAD_ARG before any device work.  Workspace functions return UINT64_MAX beyond the limits.
+ *
+ * csnappy_bc_compress        d_container[0, *d_container_length) <- exactly the bytes csnappy_bc_compress_host writes
+ *                            for (input, page_size, wm); d_in and d_container at any byte alignment; nothing is written
+ *                            at or past *d_container_length.  container_capacity >= csnappy_bc_max_container_length().
+ *                            Workspace: a fragment slot per page (csnappy_max_compressed_length(page_size) rounded up
+ *                            to 16) plus 16 bytes per page.
+ * csnappy_bc_index           *nr_pages <- the page count (written whenever it was read).  A container shorter than
+ *                            4 + 4 * nr_pages returns CSNAPPY_E_DATA_MALFORMED; index_entries < nr_pages returns
+ *                            CSNAPPY_E_BAD_ARG (index_entries 0 and d_index NULL ask for the count alone).  Else
+ *                            d_index[i] <- byte offset of page i's payload from the container start, by the index scan
+ *                            of csnappy_bc_decompress_host: the first entry above csnappy_max_compressed_length(
+ *                            page_size), or whose payload runs past container_length, and every entry behind it get
+ *                            CSNAPPY_BC_NO_PAGE.  No workspace: d_index is the scan's only memory.
+ * csnappy_bc_decompress_pages  request k decodes page d_pages[k] into d_out + k * out_stride (out_stride >=
+ *                            page_size), with d_index / nr_pages from csnappy_bc_index of the same container:
+ *                              d_status[k] 0, d_out_len[k] = bytes produced;
+ *                              or the page's decode result (what the whole-container reader reports for that page);
+ *                              or CSNAPPY_E_DATA_MALFORMED for a page whose entry is CSNAPPY_BC_NO_PAGE (or does not
+ *                              fit container_length);
+ *                              or CSNAPPY_E_BAD_ARG for a page number >= nr_pages; d_out_len[k] = 0 on failure.
+ *                            A page whose clen equals page_size is copied (a stored short last page is decoded, as in
+ *                            the host reader).  Requests may repeat and come in any order; n_requests == 0 is a no-op.
+ *                            Nothing outside [k * out_stride, k * out_stride + page_size) is written; bytes of a
+ *                            failed request are unspecified.  Workspace: 16 bytes per request + 1 KiB.
+ * csnappy_bc_decompress      *d_status, *d_out_length and *d_failed_page <- what csnappy_bc_decompress_host returns
+ *                            and writes for the same bytes (*d_out_length is 0 for the header results -5 / -2;
+ *                            *d_failed_page is written only on a page failure; it may be NULL).  Page i goes to
+ *                            d_out + i * page_size.  Workspace: 20 bytes per page for the most pages the container
+ *                            and out_capacity can hold.
+ */
+#define CSNAPPY_BC_NO_PAGE UINT64_MAX
+uint64_t csnappy_bc_compress_workspace(uint64_t input_length, uint32_t page_size);
+int csnappy_bc_compress(const void *d_in, uint64_t input_length, uint32_t page_size, void *d_container,
+			uint64_t container_capacity, uint64_t *d_container_length, int workmem_bytes_power_of_two,
+			void *d_workspace, uint64_t workspace_bytes, void *stream);
+int csnappy_bc_index(const void *d_container, uint64_t container_length, uint32_t page_size, uint64_t *d_index,
+		     uint64_t index_entries, uint32_t *nr_pages, void *stream);
+uint64_t csnappy_bc_decompress_pages_workspace(uint32_t n_requests);
+int csnappy_bc_decompress_pages(const void *d_container, uint64_t container_length, uint32_t page_size,
+				const uint64_t *d_index, uint32_t nr_pages, const uint32_t *d_pages, uint32_t n_requests,
+				void *d_out, uint64_t out_stride, uint32_t *d_out_len, int32_t *d_status,
+				void *d_workspace, uint64_t workspace_bytes, void *stream);
+uint64_t csnappy_bc_decompress_workspace(uint64_t container_length, uint32_t page_size, uint64_t out_capacity);
+int csnappy_bc_decompress(const void *d_container, uint64_t container_length, uint32_t page_size, void *d_out,
+			  uint64_t out_capacity, uint64_t *d_out_length, int32_t *d_status, uint32_t *d_failed_page,
+			  void *d_workspace, uint64_t workspace_bytes, void *stream);
 
 /*
  * Snappy FRAMING FORMAT (the format of .sz files and x-snappy-framed streams): one buffer as a stream of chunks

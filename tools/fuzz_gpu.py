@@ -5,7 +5,8 @@ also gets blocks built to drive the parse through the kernel's rare paths (tests
 sharing in stride-1 and strided windows, in-window copies, the scan end, length and offset boundaries); the decode
 leg gets random streams of every tag form (tests/streams.py), which the compressor never writes.  The container leg
 writes a page container of random page size and length, corrupts its index and payload at random and compares the
-reader with the restated reader (tests/containers.py).  The framed leg round-trips a random buffer through the framing
+reader with the restated reader (tests/containers.py), through the host call, the device-buffer reader and a random
+batch of device page reads.  The framed leg round-trips a random buffer through the framing
 format, compares the stream with the restated writer, corrupts it at random and compares the reader with the restated
 reader (tests/framed.py).  The batched-framed leg writes several random buffers in one csnappy_framed_batch_compress
 call, corrupts some of the streams, and reads valid and hostile streams together in one csnappy_framed_batch_decompress
@@ -28,13 +29,14 @@ import containers
 import framed
 from cases import fuzz_pages
 from streams import random_stream
+from test_gpu_bc_device import restated_index, restated_request
 
 budget = float(sys.argv[1]) if len(sys.argv) > 1 else 120.0
 seed = int(sys.argv[2]) if len(sys.argv) > 2 else 20261017
 chk = oracle.best()
 rng = np.random.default_rng(seed)
 t0 = time.time()
-rounds = blocks = streams = pages_read = framed_streams = batch_framed = 0
+rounds = blocks = streams = pages_read = pages_requested = framed_streams = batch_framed = 0
 while time.time() - t0 < budget:
     size = int(rng.choice([17, 64, 300, 1000, 4096, 4096, 4096, 5000, 16384, 32768]))
     wm = int(rng.integers(9, 17))
@@ -131,6 +133,32 @@ while time.time() - t0 < budget:
     assert (rc, olen, bad) == want.key(), ("container read", page, len(data), want.key(), (rc, olen, bad))
     for i, b in want.pages.items():
         assert out[i * page: i * page + len(b)].tobytes() == b, ("container page", page, i)
+    # the same broken container in device memory: the whole-container reader, then a random batch of page reads
+    d_b = torch.frombuffer(bytearray(broken), dtype=torch.uint8).cuda()
+    d_out, res = cs.api.bc_decompress_device(d_b, len(broken), page, nr * page)
+    torch.cuda.synchronize()
+    r = res.cpu().tolist()
+    assert (r[1], r[0], None if r[2] == -1 else r[2]) == want.key(), ("device container read", page, want.key(), r)
+    out = d_out.cpu().numpy()
+    for i, b in want.pages.items():
+        assert out[i * page: i * page + len(b)].tobytes() == b, ("device container page", page, i)
+    rc, idx, n_idx = cs.api.bc_index_device(d_b, len(broken), page)
+    assert rc == (containers.E_DATA_MALFORMED if len(broken) < 4 + 4 * nr else 0), ("index", rc)
+    if rc == 0:
+        offs = restated_index(bytes(broken), page)[1]
+        assert [int(x) & (2**64 - 1) for x in idx[:n_idx].cpu().tolist()] == offs, ("index", page)
+        req = rng.integers(0, nr + 2, int(rng.integers(1, 200))).astype(np.uint32)
+        stride = page + int(rng.choice([0, 0, 5, 16]))
+        o, ol, st = cs.api.bc_decompress_pages_device(d_b, idx, n_idx, torch.from_numpy(req.view(np.int32)).cuda(), page,
+                                                      len(broken), out_stride=stride)
+        torch.cuda.synchronize()
+        o, ol, st = o.cpu().numpy(), ol.cpu().tolist(), st.cpu().tolist()
+        for k, p in enumerate(req.tolist()):
+            rc_k, b = restated_request(bytes(broken), page, offs, p, nr)
+            assert (st[k], ol[k]) == (rc_k, len(b) if b is not None else 0), ("page read", page, p, st[k], rc_k)
+            if b is not None:
+                assert o[k * stride:k * stride + len(b)].tobytes() == b, ("page read bytes", page, p)
+        pages_requested += len(req)
     pages_read += nr
     # framed: a random buffer round-trips and its stream equals the restated writer; random corruptions of it give the
     # restated reader's (rc, out_length, failed_offset) and valid prefix
@@ -175,6 +203,6 @@ cs.set_tuning("decompress_lanes", 0)
 cs.set_tuning("compress_stage_input", 0)
 cs.set_tuning("decompress_stage_input", 0)
 print(f"fuzz ok: {rounds} rounds, {blocks} blocks compressed byte-identically, {streams} streams decoded with identical results, "
-      f"{pages_read} container pages written and read as restated, "
+      f"{pages_read} container pages written and read as restated, {pages_requested} device page reads as restated, "
       f"{framed_streams} framed streams written, corrupted and read as restated, "
       f"{batch_framed} streams through the batched framed calls in {time.time() - t0:.0f} s")
